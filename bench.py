@@ -2,7 +2,7 @@
 """Benchmark of the CFP fusion + cross-zone propagation path (BASELINE.json metric:
 "CFP fusion frames/s @416x544, 8x8 zones").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl cfp|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl cfp|reference] [--dump-outputs DIR]
 
 One *step* = one pass of the hot path (histogram encoder + the three TransformerFusion
 calls) over one batch of synthetic frames.  Workload = BASELINE.json configs[2]:
@@ -12,6 +12,10 @@ data-path collective (weak scaling); the time is the max over ranks.
 
 ``--impl reference`` times the reference's CPU algorithm (the oracle port of the PyTorch
 modules, oracle/cfp_oracle.py) on the host cores, on a bounded sample of the same workload.
+
+``--dump-outputs DIR`` writes what the last timed step returned (rank 0's fused maps) as float32
+DIR/fused3.npy, fused2.npy, fused1.npy, so that two builds can be compared output for output:
+the inputs, weights and positional-encoding crops are seeded, identical from run to run.
 """
 from __future__ import annotations
 
@@ -37,6 +41,24 @@ GEOMETRY = "G416"
 FLOP_PER_FRAME = 13.22e9
 DENSE_FLOP_PER_FRAME = 11.26e9
 ELEMS_PER_FRAME = 15.43e6
+DUMP_BYTES = 64 * 10**6             # --dump-outputs: every file together, .npy headers included
+
+
+def dump_outputs(out_dir, named):
+    """Write each (name, tensor) as float32 ``out_dir/<name>.npy``.  When the arrays together exceed DUMP_BYTES, every
+    one is cut to the same share of its elements: flat positions drawn by a fixed seed, in increasing order (a 1-D
+    array), so that runs with the same arguments store the same positions."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(t.numel() for _, t in named)
+    share = min(1.0, (DUMP_BYTES - 1024 * len(named)) / (4 * total))
+    for name, t in named:
+        t = t.detach().float().cpu()
+        if share < 1.0:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[: int(t.numel() * share)]
+            t = t.reshape(-1)[idx.sort().values]
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+    return share
 
 
 def load_peaks():
@@ -350,7 +372,7 @@ def run_cfp(a):
             ms0 = torch.cuda.memory_stats(dev)
             e0.record()
             for i in range(a.steps):
-                step(i)
+                outs = step(i)
                 marks[i].record()           # per-step marks (diagnostic)
                 if sampler and i == a.steps // 2:
                     sampler.sample_now()    # one clock sample while the GPU is busy with the queued steps
@@ -372,6 +394,8 @@ def run_cfp(a):
             perturbed = max_over_ranks(1.0 if max(step_ms) > 1.6 * statistics.median(step_ms) else 0.0)
             if not perturbed:
                 break
+        # the last timed step's result, copied before the replays below can overwrite a graph's output buffers
+        last_outs = [o.clone() for o in outs] if a.dump_outputs and rank == 0 else None
         if sampler:
             sampler.mark_end()
         clocks = sampler.finish() if sampler else None
@@ -498,6 +522,9 @@ def run_cfp(a):
         med = statistics.median(t)
         line["cpu_baseline"] = {"value": 1.0 / med, "unit": "frames/s", "cores": cores, "kind": "port",
                                 "sample": "1 frame/step, 3 warm-up + 10 timed, median, fp32 torch CPU ops on all host threads"}
+    if last_outs:
+        share = dump_outputs(a.dump_outputs, list(zip(("fused3", "fused2", "fused1"), last_outs)))
+        print(f"--dump-outputs: step {a.steps - 1} written to {a.dump_outputs} ({share:.3f} of the elements)", file=sys.stderr)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -1130,7 +1157,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--workload", default="combine1_b64", choices=["combine1_b64", "baseline_b16", "latency_480", "train_b32", "tail_b16"],
                     help="combine1_b64 = the headline (BASELINE.json configs[2]); the other two are side configurations")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's fused maps to DIR/<name>.npy (float32, a seeded sample above 64 MB)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "cfp" or a.workload != "combine1_b64"):
+        ap.error("--dump-outputs serves the headline workload of --impl cfp")
     if a.batch is None:
         a.batch = {"train_b32": 32, "tail_b16": 16}.get(a.workload, 64)
     if a.workload == "tail_b16":

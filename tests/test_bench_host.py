@@ -80,6 +80,27 @@ def test_committed_bench_line_carries_the_whole_contract():
     assert c["kind"] in ("port", "reference") and c["cores"] >= 1 and c["value"] > 0 and c["unit"] == d["unit"] and c["sample"]
 
 
+def test_dump_outputs_stays_in_budget_and_repeats(tmp_path, monkeypatch):
+    """--dump-outputs: float32 files, full arrays under the budget, above it the same seeded positions on every run."""
+    import numpy as np
+    import torch
+    small = [("a", torch.arange(6, dtype=torch.bfloat16).reshape(2, 3)), ("b", torch.ones(4))]
+    assert bench.dump_outputs(str(tmp_path / "full"), small) == 1.0
+    a = np.load(tmp_path / "full" / "a.npy")
+    assert a.dtype == np.float32 and a.shape == (2, 3) and np.array_equal(a, np.arange(6).reshape(2, 3))
+    monkeypatch.setattr(bench, "DUMP_BYTES", 2 * 1024 + 4 * 3000)
+    big = [("x", torch.randn(2, 4, 500)), ("y", torch.randn(8000))]
+    for run in ("r1", "r2"):
+        share = bench.dump_outputs(str(tmp_path / run), big)
+        assert 0 < share < 1
+    total = 0
+    for name, t in big:
+        s1, s2 = np.load(tmp_path / "r1" / f"{name}.npy"), np.load(tmp_path / "r2" / f"{name}.npy")
+        assert s1.dtype == np.float32 and np.array_equal(s1, s2) and np.isin(s1, t.numpy()).all()
+        total += os.path.getsize(tmp_path / "r1" / f"{name}.npy")
+    assert total <= bench.DUMP_BYTES
+
+
 def test_reference_arm_runs_on_rank_zero_only():
     """Under torchrun the CPU arm is rank 0's job: every other rank exits 0 without work and without output."""
     import os

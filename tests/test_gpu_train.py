@@ -76,7 +76,7 @@ def test_hist_encoder_train_step_matches_reference():
     sum((o * c.float().to(DEV)).sum() for o, c in zip(outs, cts)).backward()
     torch.cuda.synchronize()
     for c_, o in zip((32, 64, 128), outs):
-        assert rel_l2(o, torch.from_numpy(z[f"out{c_}"])) <= TOL
+        check_map(o, z, f"out{c_}", "hist encoder")
     assert rel_l2(hist.grad, torch.from_numpy(z["grad_hist"])) <= TOL
     check_module(enc, z, "hist encoder")
 
