@@ -415,6 +415,11 @@ int dwconv_tc(const void* in, const void** planar_out_p, int* planar_pitch, int 
     bf16* planar_out = reinterpret_cast<bf16*>(plane_ws + in_bytes);
     *planar_out_p = planar_out;          // [B][C][H][WO]; lkpm_mlp_tc reads it in place (no transpose back)
     *planar_pitch = g.WO;
+    // refuse a map too tall for the GEMM's shared memory before anything is launched: a refused call leaves the
+    // workspace and the stream untouched
+    const uint32_t t_bytes = g.NA * g.KS * 2 * kDwN * 16, a_bytes = 2 * g.KS * g.HP * 16;
+    const size_t gemm_smem = t_bytes + 3 * (size_t)((a_bytes + 127) & ~127u) + kXchBytes + kBndBytes;
+    CFP_REQUIRE(gemm_smem <= 225 * 1024, "dwconv (tensor-core path): %zu B shared memory (H=%d too tall)", gemm_smem, H);
     {
         // plane rows per CTA: 4 (64 contiguous bytes per chunk column, 35 KB slab at L1: six CTAs per SM overlap their load
         // and store phases) - measured 0.149 ms per step against 0.189 ms with 8 rows (CFP_DW_PACK_ROWS=8 | 2 for A/B runs)
@@ -427,14 +432,11 @@ int dwconv_tc(const void* in, const void** planar_out_p, int* planar_pitch, int 
         if (int err = check_launch("dw_plane_pack")) return err;
     }
     {
-        const uint32_t t_bytes = g.NA * g.KS * 2 * kDwN * 16, a_bytes = 2 * g.KS * g.HP * 16;
-        const size_t smem = t_bytes + 3 * (size_t)((a_bytes + 127) & ~127u) + kXchBytes + kBndBytes;
-        CFP_REQUIRE(smem <= 225 * 1024, "dwconv (tensor-core path): %zu B shared memory (H=%d too tall)", smem, H);
-        if (int err = set_smem(dwconv_tc_kernel, smem)) return err;
+        if (int err = set_smem(dwconv_tc_kernel, gemm_smem)) return err;
         const int total = C * g.nX * g.NB * g.nM;
         const int grid = total < sm_count() ? total : sm_count();
         const int per = (total + grid - 1) / grid;
-        launch_pdl(dwconv_tc_kernel, (total + per - 1) / per, kDwThreads, smem, st, planes, (const bf16*)toep, shift, planar_out, B, g, per, total);
+        launch_pdl(dwconv_tc_kernel, (total + per - 1) / per, kDwThreads, gemm_smem, st, planes, (const bf16*)toep, shift, planar_out, B, g, per, total);
         if (int err = check_launch(K == 31 ? "dwconv_tc<31>" : K == 15 ? "dwconv_tc<15>" : "dwconv_tc<7>")) return err;
     }
     return 0;

@@ -25,6 +25,54 @@ def rel_l2(a: torch.Tensor, b: torch.Tensor) -> float:
     return float((a - b).norm() / b.norm().clamp_min(1e-30))
 
 
+MIN_REGION = 16          # regions with fewer tokens are reported but not bounded: their rel-L2 is too noisy to hold to a ratio
+
+
+def region_errors(out: torch.Tensor, ref: torch.Tensor, regions: dict, bulk=None) -> dict:
+    """Where an error sits.  ``out`` / ``ref``: [B, H, W, C] maps; ``regions``: name -> bool token mask [B, H, W];
+    ``bulk``: the tokens the layer actually changes (all tokens when None).
+
+    Returns ``bulk`` (rel-L2 over the bulk tokens, all channels), ``regions`` (name -> (rel-L2 over the region's tokens,
+    token count)), ``token`` (the largest ||out_t - ref_t|| over the bulk, divided by the RMS token norm of ``ref`` in the
+    token's frame) with its place ``token_at`` = (frame, row, column), and ``ratio`` (the largest region error over the
+    bulk error among regions of at least ``MIN_REGION`` tokens).  A defect confined to a few percent of the tokens moves a
+    whole-map rel-L2 by little; the same defect dominates its own region and its own tokens."""
+    o, r = out.detach().double().cpu(), ref.detach().double().cpu()
+    e2 = (o - r).pow(2).sum(-1)                                  # [B, H, W] squared error per token
+    r2 = r.pow(2).sum(-1)
+    if bulk is None:
+        bulk = torch.ones_like(e2, dtype=torch.bool)
+    bulk = bulk.cpu()
+    bulk_err = float(e2[bulk].sum().sqrt() / r2[bulk].sum().sqrt().clamp_min(1e-30))
+    rms = r2.mean(dim=(1, 2), keepdim=True).sqrt().clamp_min(1e-30)
+    tok = torch.where(bulk, e2.sqrt() / rms, torch.zeros_like(e2))
+    at = np.unravel_index(int(tok.argmax()), tuple(tok.shape))
+    regs, ratio = {}, 0.0
+    for name, m in regions.items():
+        m = m.cpu()
+        n = int(m.sum())
+        if n == 0:
+            continue
+        err = float(e2[m].sum().sqrt() / r2[m].sum().sqrt().clamp_min(1e-30))
+        regs[name] = (err, n)
+        if n >= MIN_REGION:
+            ratio = max(ratio, err / max(bulk_err, 1e-30))
+    return {"bulk": bulk_err, "regions": regs, "token": float(tok.max()), "token_at": tuple(int(v) for v in at),
+            "ratio": ratio}
+
+
+def check_regions(rep: dict, what: str, ratio: float = 3.0, token_ratio: float = 10.0) -> None:
+    """Every region of at least MIN_REGION tokens within ``ratio`` x the bulk error, every bulk token within
+    ``token_ratio`` x the bulk error; a failure names the worst regions."""
+    bulk = rep["bulk"]
+    worst = sorted(((e / max(bulk, 1e-30), name, e, n) for name, (e, n) in rep["regions"].items() if n >= MIN_REGION),
+                   reverse=True)
+    where = ", ".join(f"{name} {e:.2e} ({q:.1f}x, {n} tokens)" for q, name, e, n in worst[:5])
+    assert not worst or worst[0][0] <= ratio, f"{what}: bulk rel-L2 {bulk:.2e}; worst regions: {where}"
+    assert rep["token"] <= token_ratio * bulk, \
+        f"{what}: token {rep['token_at']} off by {rep['token']:.2e} of the frame's RMS token norm (bulk {bulk:.2e}); {where}"
+
+
 def ref_keys():
     with open(os.path.join(GOLDEN, "state_dict_keys.json")) as fh:
         return json.load(fh)

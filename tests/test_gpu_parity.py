@@ -11,7 +11,7 @@ import torch
 import cfpnet_b200
 from cfpnet_b200 import _lib, geometry, synth
 from cfpnet_b200.config import args
-from helpers import FUSION_CASES as _BASE_CASES, FUSION_CASES_Z6, FusionCase, GOLDEN, ref_keys, rel_l2
+from helpers import FUSION_CASES as _BASE_CASES, FUSION_CASES_Z6, FusionCase, GOLDEN, ref_keys, region_errors, rel_l2
 
 # 6x6 zones (the reference's training layout).  They failed on their first GPU run because cfp_twins_fwd /
 # cfp_lkpm_fwd refused the workspace (their layout assumes 64 zones, the module had sized it for 36): reproduced and
@@ -205,6 +205,11 @@ def test_same_seed_same_output_and_rng_consumption():
     assert torch.equal(state, torch.get_rng_state())
 
 
+# frame run alone vs the same frame in the B = 64 batch (bf16): 3x the largest measured rel-L2 (NVIDIA B200, 1000 W power
+# limit: 3.25e-3 over L3 / L2 / L1; the largest token 3.9x its frame's rel-L2)
+FRAME_TOL = 9.7e-3
+
+
 def test_full_batch_properties():
     """BASELINE.json config 3 size (B=64, bf16, G416): size-independent properties instead of a
     64-frame oracle run — (1) frames are independent: frame i of the batch equals the same frame run
@@ -228,8 +233,13 @@ def test_full_batch_properties():
                   for k, v in inp["patch_info"].items()}
             torch.manual_seed(2)
             one = m(x[i:i + 1], feat1[i:i + 1], mask=inp["mask"][i:i + 1].to(DEV), patch_info=pi, **kw)
-            # fp32 atomics in the attention state make the last bits order-dependent
-            assert rel_l2(one, full[i:i + 1]) <= 1e-2
+            # fp32 atomics in the attention state make the last bits order-dependent: the frame alone and the frame in the
+            # batch differ by rounding only, everywhere in the frame
+            rep = region_errors(one.permute(0, 2, 3, 1), full[i:i + 1].permute(0, 2, 3, 1), {})
+            print(f"measured frame independence L{level} frame {i}: rel-L2 {rep['bulk']:.3e} token {rep['token']:.3e}")
+            assert rep["bulk"] <= FRAME_TOL, f"L{level} frame {i}: rel-L2 {rep['bulk']:.3e}"
+            assert rep["token"] <= 10 * rep["bulk"], \
+                f"L{level} frame {i}: token {rep['token_at']} off by {rep['token']:.3e} (frame rel-L2 {rep['bulk']:.3e})"
 
 
 @pytest.mark.parametrize("graph,B", [(False, 2), (True, 2), (True, 16)])
