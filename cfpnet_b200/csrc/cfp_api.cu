@@ -324,8 +324,9 @@ CFP_API int cfp_lkpm_fwd(void* feat0, int B, int H, int W, int C, const cfp_lkpm
     cudaStream_t st = (cudaStream_t)stream;
     void* y = ws + L.tok_a;
     if (dtype == CFP_BF16) {
-        static const int tc_min = getenv("CFP_DW_TC_MIN") ? atoi(getenv("CFP_DW_TC_MIN")) : 15;   // A/B switch
-        if (w->ksize >= tc_min) {  // Toeplitz GEMM on the tensor pipe (k_dwconv_tc.cu); its planar output feeds the MLP directly
+        // k >= 15: Toeplitz GEMM on the tensor pipe (k_dwconv_tc.cu); its planar output feeds the MLP directly.  At k = 7 the
+        // Toeplitz kernel measured a wash against the stencil, which stays.
+        if (w->ksize >= 15) {
             const void* planar = nullptr;
             int pitch = 0;
             if (int e = dwconv_tc(feat0, &planar, &pitch, B, H, W, C, w->ksize, w->dw_toep, w->dw_shift, ws + L.planes, st)) return e;

@@ -463,7 +463,7 @@ template <int C> struct ChainOcc { static constexpr int CTAS = C >= 128 ? 1 : (C
 // through the provider (L2-hot) in the last epilogue.
 template <int C, int NH, bool kAttnOnly, class Q, int NT>
 __global__ void __launch_bounds__((8 * NT + 2) * 32, 1) loftr_query_tc_kernel(Q q, cfp_loftr_w w, const float* __restrict__ kv,
-                                                             const float* __restrict__ ksum, int ntiles, int spread, int kv_slots) {
+                                                             const float* __restrict__ ksum, int ntiles, int kv_slots) {
     using P = ChainTC<C>;
     using S = ChainStages<C, NH, kAttnOnly, Q, NT>;
     constexpr int KG = P::KG;
@@ -473,7 +473,6 @@ __global__ void __launch_bounds__((8 * NT + 2) * 32, 1) loftr_query_tc_kernel(Q 
     __shared__ ChainBars bars;
     __shared__ float2 ln_xch[2][NT][128];                    // LayerNorm statistics of split rows, per tile group
     __shared__ float inv_den[2][S::kGroupStationary ? 128 * NH : 1];   // 1 / (Q.Ksum + eps) per (row, head), per tile group
-    const bool gs_on = (spread & 2) == 0;                    // bit 1 of `spread`: row-stationary attention epilogue (A/B runs)
     // the attention-only chain (DAPM) stages x only: half an operand buffer per tile, and the shared memory it does not
     // ask for stays L1 - where its per-frame attention state (16 KB a group at C = 128) is read from
     constexpr size_t ABUF = kAttnOnly ? (size_t)KG * P::LBO : (size_t)P::ABUF;
@@ -484,13 +483,11 @@ __global__ void __launch_bounds__((8 * NT + 2) * 32, 1) loftr_query_tc_kernel(Q 
     float* kvs = reinterpret_cast<float*>(ring + (size_t)P::NSLOT * P::SLOT);
     float* kss = kvs + (size_t)kv_slots * (C * S::DH);
     const int tid = threadIdx.x, warp = umma::warp_idx_sync();
-    // Tiles of round `it`: group g of CTA c takes tile  it * 2 G + c * ca + g * cg.  spread = 0: (ca, cg) = (2, 1), a CTA owns
-    // two neighbouring tiles; spread = 1: (1, G), the first G tiles of a round go to the groups 0 and the next G to the groups
-    // 1 - a last round of fewer than 2 G tiles then runs one tile on (almost) every SM instead of two on half of them.
-    // A group without a tile only keeps the hand-over protocol going (arrivals, barrier), and its MMAs are not issued.
+    // Tiles of round `it`: group g of CTA c takes tile  it * 2 G + 2 c + g - a CTA owns two neighbouring tiles.  A group
+    // without a tile (the last one when ntiles is odd) only keeps the hand-over protocol going (arrivals, barrier), and its
+    // MMAs are not issued.
     const int round_tiles = 2 * (int)gridDim.x;
-    const int ca = (spread & 1) ? 1 : 2, cg = (spread & 1) ? (int)gridDim.x : 1;
-    const int first0 = (int)blockIdx.x * ca;
+    const int first0 = (int)blockIdx.x * 2;
 
     if (tid == 0) {
         for (int i = 0; i < P::NSLOT; ++i) { umma::mbar_init(&bars.full[i], 1); umma::mbar_init(&bars.empty[i], 1); }
@@ -520,9 +517,9 @@ __global__ void __launch_bounds__((8 * NT + 2) * 32, 1) loftr_query_tc_kernel(Q 
             umma::fence_after_sync();
         };
         for (int first = first0; first < ntiles; first += round_tiles) {
-            const int tile = first + grp * cg;
+            const int tile = first + grp;
             int g_first = 0;
-            if (kv_slots > 0) {                              // (never with spread rounds: the pair's rows are contiguous)
+            if (kv_slots > 0) {
                 const int64_t r_first = (int64_t)first * 128;
                 const int64_t r_last = r_first + 255 < q.rows ? r_first + 255 : q.rows - 1;
                 g_first = q.group_of_row(r_first);
@@ -548,8 +545,7 @@ __global__ void __launch_bounds__((8 * NT + 2) * 32, 1) loftr_query_tc_kernel(Q 
             hand_over();
             CFP_CHAIN_MARK(2, dbg_it);
             if constexpr (S::kGroupStationary) {
-                if (gs_on) S::epi_attention_gs(q, r, tmem, wq, tid_g, a0, kv, ksum, half, &inv_den[grp][0], row0, warp % RW, RW, group_sync);
-                else S::epi_attention(q, r, tmem, wq, tid_g, a0, kv, ksum, 0, half);
+                S::epi_attention_gs(q, r, tmem, wq, tid_g, a0, kv, ksum, half, &inv_den[grp][0], row0, warp % RW, RW, group_sync);
             } else if (kv_slots > 0) {
                 umma::mbar_wait(&bars.kv_full, kvph); kvph ^= 1;
                 S::epi_attention(q, r, tmem, wq, tid_g, a0, kvs, kss, g_first, half);
@@ -604,7 +600,7 @@ __global__ void __launch_bounds__((8 * NT + 2) * 32, 1) loftr_query_tc_kernel(Q 
         };
         auto wait_a = [&]() { umma::mbar_wait(&bars.a_ready, ph); ph ^= 1; umma::fence_after_sync(); };
         for (int first = first0; first < ntiles; first += round_tiles) {
-            nlive = first + cg < ntiles ? 2 : 1;
+            nlive = first + 1 < ntiles ? 2 : 1;
             wait_a();
             block(0, 0, false);                            // q
             umma::commit(&bars.acc_ready);
@@ -790,17 +786,11 @@ __global__ void __launch_bounds__(128 * NT, MonoOcc<C>::CTAS) loftr_query_mono_k
     }
 }
 
-// threads per token row: two at C >= 64 (see ChainStages); CFP_CHAIN_NT=1 forces the thread-per-row kernels (A/B measurements)
-template <int C> struct ChainNT { static constexpr int NT = C >= 64 ? 2 : 1; };
-static bool chain_split_rows() {
-    static const bool v = [] { const char* e = getenv("CFP_CHAIN_NT"); return !(e && e[0] == '1'); }();
-    return v;
-}
-
-template <int C, int NH, bool kAttnOnly, class Q, int NT>
-static int run_query_tc_nt(const char* name, const Q& q, const cfp_loftr_w& w, const float* kv, const float* ksum,
-                           cudaStream_t st) {
+template <int C, int NH, bool kAttnOnly, class Q>
+static int run_query_tc(const char* name, const Q& q, const cfp_loftr_w& w, const float* kv, const float* ksum,
+                        cudaStream_t st) {
     using P = ChainTC<C>;
+    constexpr int NT = C >= 64 ? 2 : 1;      // threads per token row (see ChainStages): two win by 10-17 % at C >= 64
     CFP_REQUIRE(w.tc != nullptr, "%s: bf16 path needs the packed tensor-core weights (cfp_loftr_w.tc)", name);
     const int64_t ntiles = (q.rows + 127) / 128;
     CFP_REQUIRE(q.rows < ((int64_t)1 << 31), "%s: %lld rows exceed the 32-bit row index", name, (long long)q.rows);
@@ -812,7 +802,7 @@ static int run_query_tc_nt(const char* name, const Q& q, const cfp_loftr_w& w, c
         const uint32_t rpg = q.rows_per_group();
         int kv_slots = (int)((128 + rpg - 2) / rpg + 1);
         const size_t kv_bytes = (size_t)kv_slots * (C * DH + C) * sizeof(float);
-        if ((smem0 + kv_bytes + 1024) * per_sm > 227 * 1024 || getenv("CFP_NO_KV_SMEM")) kv_slots = 0;
+        if ((smem0 + kv_bytes + 1024) * per_sm > 227 * 1024) kv_slots = 0;
         const size_t smem = smem0 + (kv_slots > 0 ? kv_bytes : 0);
         const int grid = (int)(ntiles < sm_count() * per_sm ? ntiles : sm_count() * per_sm);
         auto k = loftr_query_mono_kernel<C, NH, kAttnOnly, Q, NT>;
@@ -828,15 +818,10 @@ static int run_query_tc_nt(const char* name, const Q& q, const cfp_loftr_w& w, c
         }
 #endif
     } else {
-        // CFP_CHAIN_SPREAD=1: the tiles of a round are spread over the SMs (one tile per CTA in a thin last round) instead of
-        // two neighbouring tiles per CTA.  Measured (B = 64, L3): GSA 0.147 -> 0.129 ms alone and 4.39 -> 4.37 ms per step with
-        // the levels on one stream, but 3.85 -> 3.91 ms with the three levels concurrent - a CTA with one tile takes 0.75 of
-        // the time of a CTA with two and still owns the SM's shared memory, so it costs SM-time the other levels could use.
-        static const bool spread = [] { const char* e = getenv("CFP_CHAIN_SPREAD"); return e && e[0] == '1'; }();
-        static const int no_gs = getenv("CFP_NO_GROUP_STATIONARY") ? 2 : 0;   // hist2image at C = 128: row-stationary apply (A/B)
+        // two neighbouring tiles per CTA, also in a thin last round: spreading that round one tile per CTA over all SMs was
+        // measured slower with the three levels concurrent (3.85 -> 3.91 ms per step)
         const int64_t npairs = (ntiles + 1) / 2;
-        const int64_t want = spread ? ntiles : npairs;
-        const int grid = (int)(want < sm_count() ? want : sm_count());
+        const int grid = (int)(npairs < sm_count() ? npairs : sm_count());
         auto k = loftr_query_tc_kernel<C, NH, kAttnOnly, Q, NT>;
         constexpr size_t smem0 = kAttnOnly ? 2 * (size_t)P::KG * P::LBO + (size_t)P::NSLOT * P::SLOT : P::SMEM;
         // shared-memory copy of the group states a tile pair (256 consecutive rows) touches, where it fits (groups of a frame)
@@ -844,10 +829,10 @@ static int run_query_tc_nt(const char* name, const Q& q, const cfp_loftr_w& w, c
         const uint32_t rpg = q.rows_per_group();
         int kv_slots = (int)((256 + rpg - 2) / rpg + 1);
         const size_t kv_bytes = (size_t)kv_slots * (C * DH + C) * sizeof(float);
-        if (spread || smem0 + kv_bytes + 1024 > 227 * 1024 || getenv("CFP_NO_KV_SMEM")) kv_slots = 0;
+        if (smem0 + kv_bytes + 1024 > 227 * 1024) kv_slots = 0;
         const size_t smem = smem0 + (kv_slots > 0 ? kv_bytes : 0);
         if (int e = set_smem(k, smem)) return e;
-        launch_pdl(k, grid, (8 * NT + 2) * 32, smem, st, q, w, kv, ksum, (int)ntiles, (int)spread | no_gs, kv_slots);
+        launch_pdl(k, grid, (8 * NT + 2) * 32, smem, st, q, w, kv, ksum, (int)ntiles, kv_slots);
 #ifdef CFP_DEBUG_TIMING
         {
             cudaStreamSynchronize(st);
@@ -859,15 +844,6 @@ static int run_query_tc_nt(const char* name, const Q& q, const cfp_loftr_w& w, c
 #endif
     }
     return check_launch(name);
-}
-
-template <int C, int NH, bool kAttnOnly, class Q>
-static int run_query_tc(const char* name, const Q& q, const cfp_loftr_w& w, const float* kv, const float* ksum,
-                        cudaStream_t st) {
-    if constexpr (ChainNT<C>::NT == 2) {
-        if (chain_split_rows()) return run_query_tc_nt<C, NH, kAttnOnly, Q, 2>(name, q, w, kv, ksum, st);
-    }
-    return run_query_tc_nt<C, NH, kAttnOnly, Q, 1>(name, q, w, kv, ksum, st);
 }
 
 // =====================================================================================

@@ -24,8 +24,6 @@
 #include "cfp_common.cuh"
 #include "cfp_internal.h"
 #include "umma.cuh"
-#include <cuda.h>          // CUtensorMap (types only; the encoder is fetched through cudaGetDriverEntryPoint)
-#include <stdlib.h>
 #include <stdio.h>
 
 namespace cfp {
@@ -228,244 +226,6 @@ __global__ void __launch_bounds__(192) conv3x3_tc_kernel(const bf16* __restrict_
     }
 }
 
-// ---------------------------------------------------------------------------------------
-// Same implicit GEMM with the raster brought in by the tensor-map TMA engine (cp.async.bulk.tensor, SASS UTMALDG):
-// a token-major map [B][H][W][C] is described to the TMA unit as the 5-D tensor
-//     (8 channels of a group, x, y, channel group, frame)     strides (2, 2C, 2WC, 16, 2HWC) bytes
-// and ONE box (8, W + 2, R + 2, C / 8, 1) anchored at (0, -1, y0 - 1, 0, b) lands in shared memory as
-// [channel group][raster cell][16 B] - exactly the K-major UMMA operand layout of the kernel above - with the halo
-// columns / rows outside the image zero-filled by the engine.  One elected lane issues it; the 128 row threads no longer
-// compute ~40 addresses each and wait on their own cp.async groups, they only run the epilogue (and, for the message-map
-// source, clear the cells inside the zone rectangle - that map is written outside the rectangle only,
-// transformer.py:233-234).  The operand rows a tile reads before / beyond its channel group's block (cell -1 of tap
-// (0,0); up to W + 3 cells past the block for the last tile) belong to junk output cells that the epilogue drops.
-struct ConvTmaBars {
-    uint64_t full[3], empty[3], a_full[2], a_zeroed, a_free, acc_ready;
-    uint32_t tmem_slot;
-};
-
-__device__ __forceinline__ void tma_load_5d(void* smem_dst, const CUtensorMap* tm, int c0, int c1, int c2, int c3, int c4, uint64_t* mbar) {
-    asm volatile(
-        "cp.async.bulk.tensor.5d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5, %6}], [%7];\n" ::"r"(
-            umma::smem_u32(smem_dst)),
-        "l"(tm), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4), "r"(umma::smem_u32(mbar))
-        : "memory");
-}
-
-template <int C, int TCOLS>
-__global__ void __launch_bounds__(192) conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant__ CUtensorMap tm1,
-                                                          int nsrc, const bf16* __restrict__ wpk, const float* __restrict__ shift,
-                                                          const bf16* __restrict__ residual, bf16* __restrict__ out,
-                                                          int H, int W, int R, unsigned wp_magic, int zy0, int zy1, int zx0, int zx1) {
-    using P = ConvTC<C, TCOLS>;
-    extern __shared__ __align__(128) uint8_t smem[];
-    __shared__ ConvTmaBars bars;
-    const int WP = W + 2, cells = (R + 2) * WP;
-    const uint32_t lbo_a = (uint32_t)cells * 16;
-    const uint32_t a_bytes = (uint32_t)P::KG * lbo_a;
-    uint8_t* a_buf = smem + 128;                             // one cell of slack in front (tap (0,0) of output cell 0)
-    uint8_t* ring = a_buf + ((a_bytes + (uint32_t)(WP + 4) * 16 + 127) & ~127u);   // slack behind: the last tile's junk rows
-    const int tid = threadIdx.x, warp = umma::warp_idx_sync(), lane = tid & 31;
-    const int b = blockIdx.y, y0 = blockIdx.x * R;
-    const size_t frame = (size_t)b * H * W;
-
-    if (tid == 0) {
-        for (int i = 0; i < P::NSLOT; ++i) { umma::mbar_init(&bars.full[i], 1); umma::mbar_init(&bars.empty[i], 1); }
-        umma::mbar_init(&bars.a_full[0], 1);
-        umma::mbar_init(&bars.a_full[1], 1);
-        umma::mbar_init(&bars.a_zeroed, 128);
-        umma::mbar_init(&bars.a_free, 1);
-        umma::mbar_init(&bars.acc_ready, 1);
-        umma::fence_mbar_init();
-    }
-    if (warp == 4) umma::tmem_alloc(&bars.tmem_slot, TCOLS);
-    umma::fence_before_sync();
-    __syncthreads();
-    umma::fence_after_sync();
-    const uint32_t tmem = bars.tmem_slot;
-
-    if (warp < 4) {
-        pdl_wait();
-        if (nsrc > 1) {
-            // message-map source: once its box has landed, clear the cells inside the zone rectangle
-            umma::mbar_wait(&bars.a_full[1], 0);
-            const int pr0 = max(zy0 - (y0 - 1), 0), pr1 = min(zy1 - (y0 - 1), R + 2), rw = zx1 - zx0;
-            if (pr1 > pr0 && rw > 0) {
-                const int n = (pr1 - pr0) * rw * P::KG;
-                for (int i = tid; i < n; i += 128) {
-                    const int kg = i % P::KG, j = i / P::KG, pr = pr0 + j / rw, px = zx0 + 1 + j % rw;
-                    *reinterpret_cast<uint4*>(a_buf + (size_t)kg * lbo_a + (size_t)(pr * WP + px) * 16) = make_uint4(0u, 0u, 0u, 0u);
-                }
-            }
-            umma::fence_async_smem();
-            asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];\n" ::"r"(umma::smem_u32(&bars.a_zeroed)) : "memory");
-        }
-        // ---------------- epilogue: thread = accumulator row = output cell of the padded raster (as above)
-        auto cell_of = [&](int t, bool& live) -> size_t {
-            const int o = t * 128 + warp * 32 + lane;
-            const int r = (int)__umulhi((unsigned)o, wp_magic), px = o - r * WP;   // o / WP (exact: o*WP < 2^32)
-            const int y = y0 + r, x = px - 1;
-            live = r < R && y < H && x >= 0 && x < W;
-            return (frame + (size_t)y * W + x) * C;
-        };
-        constexpr int NCH = C / 8;
-        uint4 res_next[NCH];
-        auto fetch_res = [&](int t) {
-            bool live;
-            const size_t off = cell_of(t, live);
-#pragma unroll
-            for (int k = 0; k < NCH; ++k)
-                res_next[k] = (residual && live) ? *reinterpret_cast<const uint4*>(residual + off + k * 8) : make_uint4(0u, 0u, 0u, 0u);
-        };
-        fetch_res(0);
-        umma::mbar_wait(&bars.acc_ready, 0);
-        umma::fence_after_sync();
-#pragma unroll 1
-        for (int t = 0; t < P::T; ++t) {
-            bool live;
-            const size_t off = cell_of(t, live);
-            uint4 res[NCH];
-#pragma unroll
-            for (int k = 0; k < NCH; ++k) res[k] = res_next[k];
-            if (t + 1 < P::T) fetch_res(t + 1);
-#pragma unroll
-            for (int c0 = 0; c0 < C; c0 += 16) {
-                float v[16];
-                umma::tmem_ld16(umma::tmem_addr(tmem, warp * 32, t * C + c0), v);   // warp-collective
-                if (live) {
-#pragma unroll
-                    for (int j = 0; j < 16; j += 4) {
-                        const float4 sh = *reinterpret_cast<const float4*>(shift + c0 + j);
-                        v[j] += sh.x; v[j + 1] += sh.y; v[j + 2] += sh.z; v[j + 3] += sh.w;
-                    }
-#pragma unroll
-                    for (int h = 0; h < 2; ++h) {
-                        const uint4 rr = res[(c0 >> 3) + h];
-                        const uint32_t w4[4] = {rr.x, rr.y, rr.z, rr.w};
-                        uint4 u;
-                        uint32_t* up = &u.x;
-#pragma unroll
-                        for (int k = 0; k < 4; ++k)
-                            up[k] = umma::pack_bf16(v[8 * h + 2 * k] + __uint_as_float(w4[k] << 16),
-                                                    v[8 * h + 2 * k + 1] + __uint_as_float(w4[k] & 0xffff0000u));
-                        *reinterpret_cast<uint4*>(out + off + c0 + 8 * h) = u;
-                    }
-                }
-            }
-        }
-        umma::fence_before_sync();
-    } else if (warp == 4) {
-        // ---------------- producer: the weight ring (bulk copies) and the two raster boxes (tensor-map TMA)
-        const int nchunk = nsrc * 9;
-        for (int c = 0; c < nchunk; ++c) {
-            const int slot = c % P::NSLOT, round = c / P::NSLOT;
-            if (round > 0) umma::mbar_wait(&bars.empty[slot], (round - 1) & 1);
-            umma::bulk_load(ring + (size_t)slot * P::SLOT_BYTES, wpk + (size_t)c * C * C, P::SLOT_BYTES, &bars.full[slot]);
-            if (c == P::NSLOT - 1 || c == 9) {               // first weight blocks on their way -> source 0; source 1 once
-                const int s = c == 9 ? 1 : 0;                //   every MMA reading source 0 has completed
-                if (s == 0) pdl_wait();                      // the maps come from the previous kernels of the stream
-                else umma::mbar_wait(&bars.a_free, 0);
-                if (umma::elect_one()) {
-                    umma::mbar_expect_tx(&bars.a_full[s], a_bytes);
-                    tma_load_5d(a_buf, s == 0 ? &tm0 : &tm1, 0, -1, y0 - 1, 0, b, &bars.a_full[s]);
-                }
-                __syncwarp();
-            }
-        }
-    } else {
-        // ---------------- MMA issuer (whole warp runs the loop; one elected lane issues)
-        const uint32_t idesc = umma::idesc_bf16(128, C);
-        const uint32_t a0 = umma::smem_u32(a_buf), w0 = umma::smem_u32(ring);
-        constexpr uint32_t lbo_b = C * 16;
-        int c = 0;
-        for (int s = 0; s < nsrc; ++s) {
-            umma::mbar_wait(&bars.a_full[s], 0);
-            if (s == 1) umma::mbar_wait(&bars.a_zeroed, 0);
-            umma::fence_after_sync();
-            for (int tap = 0; tap < 9; ++tap, ++c) {
-                const int slot = c % P::NSLOT, round = c / P::NSLOT;
-                umma::mbar_wait(&bars.full[slot], round & 1);
-                umma::fence_after_sync();
-                const int tap_cell = (tap / 3) * WP + (tap % 3) - 1;
-                const uint64_t wd0 = umma::smem_desc(w0 + slot * P::SLOT_BYTES, lbo_b);
-                uint64_t ad0 = umma::smem_desc((uint32_t)((int)a0 + tap_cell * 16), lbo_a);
-#pragma unroll 1
-                for (int t = 0; t < P::T; ++t) {
-                    uint64_t ad = ad0, wd = wd0;
-#pragma unroll
-                    for (int ks = 0; ks < C / 16; ++ks) {
-                        umma::mma_bf16(tmem + t * C, ad, wd, idesc, (c | ks) != 0);
-                        ad = umma::desc_advance(ad, 2 * lbo_a);
-                        wd = umma::desc_advance(wd, 2 * lbo_b);
-                    }
-                    ad0 = umma::desc_advance(ad0, 128 * 16);
-                }
-                umma::commit(&bars.empty[slot]);
-            }
-            umma::commit(s + 1 < nsrc ? &bars.a_free : &bars.acc_ready);
-        }
-    }
-    pdl_trigger();                         // this CTA's work is done: the next kernel of the stream may start its prologue
-    __syncthreads();
-    if (warp == 4) {
-        umma::fence_after_sync();
-        umma::tmem_dealloc(tmem, TCOLS);
-    }
-}
-
-// cuTensorMapEncodeTiled through the runtime (no link against libcuda)
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_tiled_fn() {
-    static EncodeTiledFn fn = [] {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess)
-            p = nullptr;
-        return (EncodeTiledFn)p;
-    }();
-    return fn;
-}
-// token-major bf16 map [B][H][W][C] as (8 ch, x, y, channel group, frame), box = (8, W + 2, rows, C / 8, 1)
-static int raster_tensor_map(CUtensorMap* tm, const void* base, int B, int H, int W, int C, int box_rows) {
-    EncodeTiledFn enc = encode_tiled_fn();
-    CFP_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled is not available from this driver");
-    const cuuint64_t gdim[5] = {8, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)(C / 8), (cuuint64_t)B};
-    const cuuint64_t gstr[4] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, 16, (cuuint64_t)H * W * C * 2};
-    const cuuint32_t box[5] = {8, (cuuint32_t)(W + 2), (cuuint32_t)box_rows, (cuuint32_t)(C / 8), 1};
-    const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    const CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(base), gdim, gstr, box, estr,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    CFP_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed (%d) for a [%d][%d][%d][%d] map, box rows %d", (int)r, B, H, W, C, box_rows);
-    return 0;
-}
-
-template <int C, int TCOLS>
-static int conv_tma_launch(const void* in0, const void* in1, const void* wpk, const float* shift, const void* residual,
-                           void* out, int B, int H, int W, int zy0, int zy1, int zx0, int zx1, cudaStream_t st) {
-    using P = ConvTC<C, TCOLS>;
-    const int WP = W + 2;
-    const int R = (P::T * 128) / WP;
-    CFP_REQUIRE(R >= 1 && WP <= 256 && R + 2 <= 256, "conv3x3 (tensor-core path): map width %d exceeds %d", W, P::T * 128 - 2 < 254 ? P::T * 128 - 2 : 254);
-    const size_t a_bytes = (size_t)P::KG * (R + 2) * WP * 16;
-    const size_t smem = 128 + ((a_bytes + (size_t)(WP + 4) * 16 + 127) & ~(size_t)127) + (size_t)P::NSLOT * P::SLOT_BYTES;
-    CFP_REQUIRE(smem <= 220 * 1024, "conv3x3 (tensor-core path): %zu B shared memory", smem);
-    CFP_REQUIRE((((uintptr_t)in0 | (uintptr_t)in1) & 15) == 0, "conv3x3: maps must be 16-byte aligned");
-    CUtensorMap tm0, tm1;
-    if (int e = raster_tensor_map(&tm0, in0, B, H, W, C, R + 2)) return e;
-    if (int e = raster_tensor_map(&tm1, in1 ? in1 : in0, B, H, W, C, R + 2)) return e;
-    auto k = conv3x3_tma_kernel<C, TCOLS>;
-    if (int e = set_smem(k, smem)) return e;
-    dim3 grid((H + R - 1) / R, B);
-    const unsigned wp_magic = (unsigned)((((uint64_t)1 << 32) + WP - 1) / WP);
-    launch_pdl(k, grid, 192, smem, st, tm0, tm1, in1 ? 2 : 1, (const bf16*)wpk, shift, (const bf16*)residual, (bf16*)out, H, W, R,
-               wp_magic, zy0, zy1, zx0, zx1);
-    return check_launch(in1 ? (C == 32 ? "conv3x3_tc<2C->C,32>" : C == 64 ? "conv3x3_tc<2C->C,64>" : "conv3x3_tc<2C->C,128>")
-                            : (C == 32 ? "conv3x3_tc<C->C,32>" : C == 64 ? "conv3x3_tc<C->C,64>" : "conv3x3_tc<C->C,128>"));
-}
-
 template <int C, int TCOLS>
 static int conv_tc_launch(const void* in0, const void* in1, const void* wpk, const float* shift, const void* residual,
                           void* out, int B, int H, int W, int zy0, int zy1, int zx0, int zx1, cudaStream_t st) {
@@ -499,41 +259,15 @@ static int conv_tc_launch(const void* in0, const void* in1, const void* wpk, con
 int conv3x3_tc(const void* in0, const void* in1, const void* wpk, const float* shift, const void* residual, void* out,
                int B, int H, int W, int C, int zy0, int zy1, int zx0, int zx1, cudaStream_t st) {
     CFP_REQUIRE(B <= 65535, "B too large for grid.y");
-    // CTA size: 256 accumulator columns (T = 256/C M-tiles, one or two CTAs per SM) or 128 (half the raster, twice the
-    // CTAs per SM: the stage -> MMA -> epilogue phases of a CTA are serial, co-resident CTAs are what overlaps them)
-    // measured (B200, 64 frames): 128 columns win for C = 32 / 64 (0.84x / 0.93x the time), 256 for C = 128
-    static const int tcols_env = getenv("CFP_CONV_TCOLS") ? atoi(getenv("CFP_CONV_TCOLS")) : 0;
-    const int tcols = tcols_env ? tcols_env : (C <= 64 ? 128 : 256);
+    // CTA size: 128 accumulator columns (T = 128/C M-tiles) at C <= 64, 256 at C = 128: with half the raster per CTA, twice
+    // the CTAs share an SM, and co-resident CTAs are what overlaps the serial stage -> MMA -> epilogue phases of a CTA.
+    // Measured (B200, 64 frames): 128 columns win for C = 32 / 64 (0.84x / 0.93x the time), 256 for C = 128.
+    // Raster staging by tensor-map TMA was measured and removed: equal at C = 64 / 128, 6 % slower at C = 32, and the
+    // cp.async form is 1.3 % faster on the concurrent step.
 #define CFP_CONV_ARGS in0, in1, wpk, shift, residual, out, B, H, W, zy0, zy1, zx0, zx1, st
-    // raster staging: per-thread zero-fill cp.async by default, tensor-map TMA (cp.async.bulk.tensor, one 5-D box per source)
-    // with CFP_CONV_TMA=1.  Measured (B200, 64 frames, both convs of a DAPM, alone on the GPU): C = 64 0.255 (TMA) vs 0.254 ms,
-    // C = 128 0.193 vs 0.189 ms - equal; C = 32 0.374 vs 0.351 ms - the box's innermost extent is one 16-byte channel group
-    // (the no-swizzle operand layout keeps a cell's groups 16 B x cells apart), so the engine fetches half-used 32-byte
-    // sectors once per group where consecutive cp.async threads cover whole lines.  With the three levels concurrent (the
-    // headline workload) the cp.async form is 1.3 % faster on the whole step (3.47 -> 3.42 ms, final build of round 2), which
-    // is why it is the default; tests/test_gpu_layers.py runs the DAPM parity cases through the TMA form in a subprocess.
-    static const int tma_env = getenv("CFP_CONV_TMA") ? atoi(getenv("CFP_CONV_TMA")) : -1;
-    const bool use_tma = tma_env >= 0 ? tma_env != 0 : false;
-    if (use_tma && W + 2 <= 256) {
-        if (tcols == 128) {
-            if (C == 32) return conv_tma_launch<32, 128>(CFP_CONV_ARGS);
-            if (C == 64) return conv_tma_launch<64, 128>(CFP_CONV_ARGS);
-            if (C == 128) return conv_tma_launch<128, 128>(CFP_CONV_ARGS);
-        } else {
-            if (C == 32) return conv_tma_launch<32, 256>(CFP_CONV_ARGS);
-            if (C == 64) return conv_tma_launch<64, 256>(CFP_CONV_ARGS);
-            if (C == 128) return conv_tma_launch<128, 256>(CFP_CONV_ARGS);
-        }
-    }
-    if (tcols == 128) {
-        if (C == 32) return conv_tc_launch<32, 128>(CFP_CONV_ARGS);
-        if (C == 64) return conv_tc_launch<64, 128>(CFP_CONV_ARGS);
-        if (C == 128) return conv_tc_launch<128, 128>(CFP_CONV_ARGS);
-    } else {
-        if (C == 32) return conv_tc_launch<32, 256>(CFP_CONV_ARGS);
-        if (C == 64) return conv_tc_launch<64, 256>(CFP_CONV_ARGS);
-        if (C == 128) return conv_tc_launch<128, 256>(CFP_CONV_ARGS);
-    }
+    if (C == 32) return conv_tc_launch<32, 128>(CFP_CONV_ARGS);
+    if (C == 64) return conv_tc_launch<64, 128>(CFP_CONV_ARGS);
+    if (C == 128) return conv_tc_launch<128, 256>(CFP_CONV_ARGS);
 #undef CFP_CONV_ARGS
     return fail("unsupported C=%d", C);
 }

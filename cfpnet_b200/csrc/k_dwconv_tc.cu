@@ -37,7 +37,6 @@
 #include "cfp_common.cuh"
 #include "cfp_internal.h"
 #include "umma.cuh"
-#include <stdlib.h>
 
 namespace cfp {
 
@@ -422,11 +421,11 @@ int dwconv_tc(const void* in, const void** planar_out_p, int* planar_pitch, int 
     CFP_REQUIRE(gemm_smem <= 225 * 1024, "dwconv (tensor-core path): %zu B shared memory (H=%d too tall)", gemm_smem, H);
     {
         // plane rows per CTA: 4 (64 contiguous bytes per chunk column, 35 KB slab at L1: six CTAs per SM overlap their load
-        // and store phases) - measured 0.149 ms per step against 0.189 ms with 8 rows (CFP_DW_PACK_ROWS=8 | 2 for A/B runs)
-        static const int rpc = [] { const char* e = getenv("CFP_DW_PACK_ROWS"); return e && e[0] == '8' ? 8 : (e && e[0] == '2' ? 2 : 4); }();
+        // and store phases) - measured 0.149 ms per step against 0.189 ms with 8 rows
+        constexpr int rpc = 4;
         const size_t smem = (size_t)rpc * dw_slab_row_words(W, C) * 4;
         CFP_REQUIRE(smem <= 200 * 1024, "dw_plane_pack: %zu B shared memory", smem);
-        auto kp = rpc == 4 ? dw_plane_pack_kernel<4> : (rpc == 2 ? dw_plane_pack_kernel<2> : dw_plane_pack_kernel<8>);
+        auto kp = dw_plane_pack_kernel<rpc>;
         if (int err = set_smem(kp, smem)) return err;
         launch_pdl(kp, dim3((g.HP + rpc - 1) / rpc, g.NB), 256, smem, st, (const bf16*)in, planes, g, B);
         if (int err = check_launch("dw_plane_pack")) return err;

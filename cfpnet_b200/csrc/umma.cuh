@@ -156,29 +156,14 @@ __device__ __forceinline__ void mbar_expect_tx(uint64_t* mbar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"(smem_u32(mbar)), "r"(bytes) : "memory");
 }
 // try_wait is potentially blocking: the hardware may suspend the thread until the phase completes or a time limit
-// passes.  Without a hint that limit is short and a waiting warp comes back to re-issue try_wait + branch every few
-// hundred cycles; every kernel here has 4-16 row warps waiting on an accumulator while ONE warp must get issue slots to
-// feed the tensor pipe (and service warps polling empty / full barriers next to epilogue warps).  Telling the waiters
-// to sleep (CFP_MBAR_HINT_NS > 0) was MEASURED and is off: with a 1 ms hint the step went 4.05 -> 4.09 ms
-// (lkpm_mlp_tc<32> +12 %, the others unchanged): the wake-up after a suspended wait costs more than the polling.
-#ifndef CFP_MBAR_HINT_NS
-#define CFP_MBAR_HINT_NS 0
-#endif
+// passes.  A suspend-time hint was measured slower (step 4.05 -> 4.09 ms): the wake-up costs more than the polling.
 __device__ __forceinline__ bool mbar_try_wait(uint64_t* mbar, uint32_t parity) {
     uint32_t ok;
-#if CFP_MBAR_HINT_NS > 0
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
-        : "=r"(ok)
-        : "r"(smem_u32(mbar)), "r"(parity), "r"((uint32_t)CFP_MBAR_HINT_NS)
-        : "memory");
-#else
     asm volatile(
         "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
         : "=r"(ok)
         : "r"(smem_u32(mbar)), "r"(parity)
         : "memory");
-#endif
     return ok != 0;
 }
 __device__ __forceinline__ void mbar_wait(uint64_t* mbar, uint32_t parity) {

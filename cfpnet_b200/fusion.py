@@ -22,19 +22,6 @@ from .layers import Combine1, LoFTREncoderLayer, TwinsTransformer
 from .packing import PackCache, Packer, Scratch, host, relocate
 
 
-MICRO_DEFAULT = {128: 1, 64: 1, 32: 1}
-
-
-def _micro_default(dim: int) -> int:
-    import os
-    table = dict(MICRO_DEFAULT)
-    for item in os.environ.get("CFP_MICRO", "").split(","):
-        if ":" in item:
-            k, v = item.split(":")
-            table[int(k)] = int(v)
-    return max(1, table.get(dim, 1))
-
-
 class TransformerFusion(nn.Module):
     def __init__(self, embedding_dim, max_resolution, num_heads=4, large_kernel=None, patch_size=None):
         super().__init__()
@@ -67,8 +54,6 @@ class TransformerFusion(nn.Module):
         self.conv_patch_size = 640 / self.max_resolution[1]
         self._cache = PackCache()
         self._scratch = Scratch()
-        # batch slices run on separate streams inside one forward (see forward()); CFP_MICRO="128:4,64:2,32:1" overrides
-        self.micro_batches = _micro_default(embedding_dim)
 
     def _replicate_for_data_parallel(self):
         """``nn.DataParallel`` replicas copy ``__dict__`` shallowly: give each its own pack cache and scratch (the
@@ -169,7 +154,7 @@ class TransformerFusion(nn.Module):
             lib = _lib.load()
             ws_bytes = lib.cfp_workspace_bytes(B, H, W, D, self.ws, self.large_kernel or 0, code, C.byref(cg))
             work, feat0 = self._scratch.get(
-                dev.index, (dt, B, H, W, 0), lambda t: t[0].numel() >= ws_bytes,
+                dev.index, (dt, B, H, W), lambda t: t[0].numel() >= ws_bytes,
                 lambda: (torch.empty(ws_bytes, device=dev, dtype=torch.uint8), torch.empty(B, H * W, D, device=dev, dtype=dt)))
             st = _lib.stream_ptr()
             _lib.call("cfp_posenc_tokens_nhwc_fwd", x_tok.data_ptr(), x_pitch, pos, feat0.data_ptr(), B, D, H, W,
@@ -255,61 +240,25 @@ class TransformerFusion(nn.Module):
             raise ValueError("out= must be a contiguous tensor shaped and typed like x")
         emb_copy = (not args.change_embedding) and "hist2image" in self.layer_names
 
-        def run(part, b0, b1):
-            """Frames [b0, b1) through the layer list on the current stream (scratch slot `part`)."""
-            Bp = b1 - b0
+        with torch.cuda.device(dev):
             lib = _lib.load()
-            ws_bytes = lib.cfp_workspace_bytes(Bp, H, W, D, self.ws, self.large_kernel or 0, code, C.byref(cg))
+            ws_bytes = lib.cfp_workspace_bytes(B, H, W, D, self.ws, self.large_kernel or 0, code, C.byref(cg))
             # scratch (workspace + token map) is owned by the module and reused across calls: stream order
             # makes that safe for back-to-back forwards on one stream, and it keeps hundreds of MB of
             # per-call allocations (cudaMalloc stalls once several streams are in play) off the hot path.
             # One module instance must not run on two streams at once (replicas own their scratch).
             work, feat0 = self._scratch.get(
-                dev.index, (dt, Bp, H, W, part), lambda t: t[0].numel() >= ws_bytes,
+                dev.index, (dt, B, H, W), lambda t: t[0].numel() >= ws_bytes,
                 lambda: (torch.empty(ws_bytes, device=dev, dtype=torch.uint8),
-                         torch.empty(Bp, H * W, D, device=dev, dtype=dt)))
+                         torch.empty(B, H * W, D, device=dev, dtype=dt)))
             st = _lib.stream_ptr()
-            xp, f1p, mp, op = x[b0:b1], feat1[b0:b1], mask[b0:b1], out[b0:b1]
             if crop_dev is not None:
-                _lib.call("cfp_posenc_tokens_crop_fwd", xp.data_ptr(), pos, feat0.data_ptr(), Bp, D, H, W,
+                _lib.call("cfp_posenc_tokens_crop_fwd", x.data_ptr(), pos, feat0.data_ptr(), B, D, H, W,
                           self.max_resolution[0], self.max_resolution[1], crop_dev.data_ptr(), code, st)
             else:
-                _lib.call("cfp_posenc_tokens_fwd", xp.data_ptr(), pos, feat0.data_ptr(), Bp, D, H, W,
+                _lib.call("cfp_posenc_tokens_fwd", x.data_ptr(), pos, feat0.data_ptr(), B, D, H, W,
                           self.max_resolution[0], self.max_resolution[1], oy, ox, code, st)
-            if not self._run_layers(packed, pos2, feat0, f1p, mp, Bp, H, W, D, S, cg, work, ws_bytes, code, st, emb_copy,
-                                    out_nchw=op):
-                _lib.call("cfp_tokens_to_nchw", feat0.data_ptr(), op.data_ptr(), Bp, D, H, W, code, st)
-
-        parts = max(1, min(int(self.micro_batches), B))
-        with torch.cuda.device(dev):
-            if parts == 1:
-                run(0, 0, B)
-                return out
-            # Frames are independent in eval mode: the batch is cut into `parts` slices that run the layer list on
-            # separate streams.  The kernels of the small maps (1/16 scale: one or two waves of long serial tile
-            # chains, one CTA per SM) are latency-bound; two half-batches keep twice as many chains in flight.
-            cur = torch.cuda.current_stream(dev)
-            side = self.__dict__.setdefault("_part_streams", {}).setdefault(
-                dev.index, [torch.cuda.Stream(dev) for _ in range(8)])
-            fork = torch.cuda.Event()
-            fork.record(cur)
-            joins = []
-            prev_pdl = _lib.set_pdl(False)       # pre-launched CTAs would only take slots from the other slices' kernels
-            try:
-                for i in range(parts):
-                    b0, b1 = i * B // parts, (i + 1) * B // parts
-                    if i == parts - 1:
-                        run(i, b0, b1)           # the last slice stays on the caller's stream
-                        continue
-                    s_ = side[i % len(side)]
-                    s_.wait_event(fork)
-                    with torch.cuda.stream(s_):
-                        run(i, b0, b1)
-                        e = torch.cuda.Event()
-                        e.record(s_)
-                    joins.append(e)
-            finally:
-                _lib.set_pdl(bool(prev_pdl))
-            for e in joins:
-                cur.wait_event(e)
+            if not self._run_layers(packed, pos2, feat0, feat1, mask, B, H, W, D, S, cg, work, ws_bytes, code, st, emb_copy,
+                                    out_nchw=out):
+                _lib.call("cfp_tokens_to_nchw", feat0.data_ptr(), out.data_ptr(), B, D, H, W, code, st)
         return out

@@ -36,8 +36,6 @@ class FusionPath(nn.Module):
         self.hist_encoder.out_dtype = dtype
         return self
 
-    # stream_host: per-input "landed" / per-level "done" events instead of one of each per batch (CFP_COARSE_EVENTS=1: the old form)
-    fine_grained_events = not bool(__import__("os").environ.get("CFP_COARSE_EVENTS"))
     # run the three fusion calls of the synthetic harness on three streams (CFP_SEQUENTIAL_LEVELS=1: one stream, the drop-in order)
     concurrent_levels = not bool(__import__("os").environ.get("CFP_SEQUENTIAL_LEVELS"))
 
@@ -197,7 +195,7 @@ class FusionPath(nn.Module):
         if (str(dev), depth) not in cache:
             cache[(str(dev), depth)] = dict(
                 h2d=torch.cuda.Stream(dev), d2h=torch.cuda.Stream(dev),
-                slots=[dict(inp=None, out=None, in_ready=torch.cuda.Event(), comp_done=torch.cuda.Event(),
+                slots=[dict(inp=None, out=None, comp_done=torch.cuda.Event(),
                             out_ready=torch.cuda.Event(), busy=False, graph=None,
                             # per-input / per-level events (external: they survive CUDA-graph capture as event nodes)
                             ready={k: torch.cuda.Event(external=True) for k in ("hist", "x3", "x2", "x1")},
@@ -223,7 +221,6 @@ class FusionPath(nn.Module):
             if sl["inp"] is None or any(sl["inp"][k].shape != hb[k].shape or sl["inp"][k].dtype != hb[k].dtype for k in keys):
                 sl["inp"] = {k: torch.empty(hb[k].shape, dtype=hb[k].dtype, device=dev) for k in keys}
                 sl["graph"] = None
-            fine = self.fine_grained_events
             with torch.cuda.stream(h2d):
                 h2d.wait_event(sl["comp_done"])          # previous compute on these input buffers finished
                 # smallest first: histograms + mask, then the 1/16, 1/8, 1/4 maps - each followed by its own event, so that a
@@ -234,10 +231,8 @@ class FusionPath(nn.Module):
                 for k in ("x3", "x2", "x1"):
                     sl["inp"][k].copy_(hb[k], non_blocking=True)
                     sl["ready"][k].record(h2d)
-                sl["in_ready"].record(h2d)
-            if not fine:
-                comp.wait_event(sl["in_ready"])
-            ev = dict(ready=sl["ready"], done=sl["done"]) if fine else {}
+            # per-input / per-level events rather than one of each per batch: measured K = 10 16.50 -> 16.92 k frames/s
+            ev = dict(ready=sl["ready"], done=sl["done"])
             if seed_it is not None:
                 torch.manual_seed(next(seed_it))
             d = sl["inp"]
@@ -253,11 +248,8 @@ class FusionPath(nn.Module):
             if sl["out"] is None or any(p.shape != o.shape or p.dtype != o.dtype for p, o in zip(sl["out"], outs)):
                 sl["out"] = [torch.empty(o.shape, dtype=o.dtype, pin_memory=True) for o in outs]
             with torch.cuda.stream(d2h):
-                if not fine:
-                    d2h.wait_event(sl["comp_done"])
                 for j, (p, o) in enumerate(zip(sl["out"], outs)):
-                    if fine:
-                        d2h.wait_event(sl["done"][j])     # this level's map is complete (the others may still be running)
+                    d2h.wait_event(sl["done"][j])         # this level's map is complete (the others may still be running)
                     p.copy_(o, non_blocking=True)
                 sl["out_ready"].record(d2h)
             # keep the device results referenced until this slot is drained (host-synchronised on out_ready):

@@ -1,7 +1,6 @@
 """Per-layer checks through the C ABI: each bf16 (tensor-core) layer entry point against the
 fp32 (exact FFMA) entry point of the same library on identical inputs, and against the oracle."""
 import ctypes
-import os
 
 import pytest
 import torch
@@ -116,33 +115,6 @@ def test_dapm_layer_vs_oracle(level):
     assert rel_l2(out, truth) <= 1e-4
 
 
-@pytest.mark.parametrize("parts", [2, 3])
-def test_micro_batched_forward_equals_whole_batch(parts):
-    """TransformerFusion.micro_batches: the batch cut into slices on separate streams gives the whole-batch result
-    (fp32: bit-identical except for the fp32 atomics of straddling attention groups)."""
-    import cfpnet_b200
-    from cfpnet_b200 import synth
-    from helpers import ref_keys, rel_l2
-    dev = "cuda:0"
-    inp = synth.make_inputs("G416", 5, seed=9, levels=(3,))
-    enc = cfpnet_b200.HistogramEncoder()
-    enc.load_state_dict(synth.synthetic_state_dict(ref_keys()["hist_encoder"], seed=0))
-    enc = enc.to(dev).eval()
-    args.attention_layer = list(synth.COMBINE1_LAYERS)
-    m = cfpnet_b200.TransformerFusion(128, [30, 40], large_kernel=7, patch_size=4)
-    m.load_state_dict(synth.synthetic_state_dict(ref_keys()["fusion_combine1_L3"], seed=3))
-    m = m.to(dev).eval()
-    outs = []
-    with torch.no_grad():
-        f128 = enc(inp["hist_data"].to(dev).unsqueeze(-1))[2]
-        for p in (1, parts):
-            m.micro_batches = p
-            torch.manual_seed(5)
-            outs.append(m(inp["x3"].to(dev), f128, mask=inp["mask"].to(dev), patch_info=inp["patch_info"], rect_data=None, rgb=None).float().cpu())
-    torch.cuda.synchronize()
-    assert rel_l2(outs[1], outs[0]) <= 1e-5
-
-
 @pytest.mark.parametrize("level,dtype", [(3, torch.bfloat16), (2, torch.bfloat16), (1, torch.bfloat16), (3, torch.float32)])
 def test_last_layer_nchw_epilogue_equals_layer_then_transpose(level, dtype):
     """cfp_twins_nchw_fwd (the GSA chain's last epilogue stores the caller's NCHW map) against cfp_twins_fwd followed by
@@ -174,16 +146,3 @@ def test_last_layer_nchw_epilogue_equals_layer_then_transpose(level, dtype):
         _lib.call("cfp_twins_nchw_fwd", x.data_ptr(), x.data_ptr(), B, H, W, C, ctypes.byref(packed[2]), work.data_ptr(), nbytes, code,
                   _lib.stream_ptr())
 
-
-def test_dapm_bf16_through_the_tensor_map_tma_staging():
-    """conv3x3_tma_kernel (raster staged by cp.async.bulk.tensor boxes) is not the default staging any more (the cp.async
-    form is 1.3 % faster on the concurrent step): the library reads CFP_CONV_TMA once per process, so the DAPM bf16-vs-fp32
-    cases of this file are run again in a child process with CFP_CONV_TMA=1 to keep that kernel under test."""
-    import subprocess
-    import sys
-    env = dict(os.environ, CFP_CONV_TMA="1")
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(root, "tests", "test_gpu_layers.py"), "-q", "-x", "-m", "gpu",
-                        "-k", "test_bf16_layer_matches_fp32_layer and dapm"], env=env, cwd=root, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    assert "3 passed" in r.stdout, r.stdout[-500:]

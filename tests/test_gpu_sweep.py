@@ -11,10 +11,6 @@ layer changes (the bulk) <= BF16_TOL[layer, level]; every region of at least 16 
 call; every token (||out_t - ref_t|| over the frame's RMS token norm) <= 10x the bulk error."""
 import ctypes
 import functools
-import os
-import re
-import subprocess
-import sys
 
 import pytest
 import torch
@@ -437,25 +433,3 @@ def test_fusion_other_image_sizes(size, level, engine, monkeypatch):
     regs = {**frame_regions(B, H, W), **tile_regions(B, H, W)}
     judge(out.permute(0, 2, 3, 1), ref.permute(0, 2, 3, 1), B, H, W, regs, "fusion", level, engine, f"fusion {size} L{level} {engine}")
 
-
-# ------------------------------------------------------------------ experiment switches
-# The library reads these once per process: each child runs the bf16 cases of the LKPM / Twins sweeps and the hand-built
-# zone layouts (every level) under its switches.  Alternatives of one kernel sit in different children.
-CHILDREN = {
-    "dw_tc_k7": {"CFP_DW_TC_MIN": "7", "CFP_DW_PACK_ROWS": "2", "CFP_CHAIN_NT": "1", "CFP_CONV_TCOLS": "128"},
-    "dw_tiles": {"CFP_DW_FRAME": "0", "CFP_DW_PACK_ROWS": "8", "CFP_NO_KV_SMEM": "1", "CFP_CONV_TCOLS": "256"},
-    "chain": {"CFP_CHAIN_SPREAD": "1", "CFP_NO_GROUP_STATIONARY": "1"},
-}
-CHILD_CASES = len(LKPM_SHAPES) + len(twins_shapes()) + len(HAND)     # bf16 cases
-
-
-@pytest.mark.parametrize("child", list(CHILDREN))
-def test_experiment_switches_change_no_result(child):
-    env = dict(os.environ, **CHILDREN[child])
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-q", "-m", "gpu", "-p", "no:cacheprovider",
-                        "-k", "bf16 and (lkpm_sweep or twins_sweep or zone_layers_hand)"],
-                       env=env, cwd=root, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
-    n = re.search(r"(\d+) passed", r.stdout)
-    assert n and int(n.group(1)) == CHILD_CASES, r.stdout[-500:]

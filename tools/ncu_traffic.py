@@ -41,7 +41,7 @@ def main(path, out):
             name = f"kv_state_tc<{kind},{t[0]}>"
         elif fn in ("loftr_query_tc_kernel", "loftr_query_mono_kernel"):
             name = (f"attn_query_tc<{kind},{t[0]}>" if t[2] == "1" else f"loftr_query_tc<{kind},{t[0]}>")
-        elif fn in ("conv3x3_tc_kernel", "conv3x3_tma_kernel"):       # same op, cp.async / tensor-map TMA raster staging
+        elif fn == "conv3x3_tc_kernel":
             level_c = t[0]
             name = f"conv3x3_tc<{'2C->C' if conv_parity == 0 else 'C->C'},{t[0]}>"
             conv_parity ^= 1
