@@ -550,6 +550,50 @@ CFP_API int cfp_head_expect(const void* x, int pitch, int B, int npix, const voi
     return head_expect_tc(x, pitch, B, npix, w_tc, bias, centres, n_bins, pred, prob, (cudaStream_t)stream);
 }
 
+// the exact fp32 engine of the same stages (k_dec_f32.cu)
+CFP_API int cfp_conv_f32_fwd(const float* in, int B, int H, int W, int cin, int cout, int ksize, const float* w, const float* shift,
+                             float leaky_slope, float* out, int out_pitch, int out_coff, void* stream) {
+    begin_call(stream);
+    CFP_REQUIRE(in && w && shift && out, "null pointer");
+    CFP_REQUIRE(ksize == 1 || ksize == 3, "kernel size %d (1 and 3 are served)", ksize);
+    return conv_f32(in, cin, ksize * ksize, w, shift, leaky_slope, out, out_pitch, out_coff, B, H, W, cout, (cudaStream_t)stream);
+}
+CFP_API int cfp_upsample_concat_f32(const float* lo, int h, int w, int c_lo, int lo_pitch, const float* skip, int c_skip, float* out, int B,
+                                    int H, int W, int c_out, void* stream) {
+    begin_call(stream);
+    CFP_REQUIRE(out, "null pointer");
+    return upsample_concat_f32(lo, h, w, c_lo, lo_pitch, skip, c_skip, out, B, H, W, c_out, (cudaStream_t)stream);
+}
+CFP_API int cfp_posenc_tokens_nhwc_f32_fwd(const float* x, int x_pitch, const float* pos, float* tokens, int B, int C, int H, int W,
+                                           int pos_h, int pos_w, int oy, int ox, void* stream) {
+    begin_call(stream);
+    CFP_REQUIRE(x && pos && tokens, "null pointer");
+    CFP_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, "bad shape");
+    CFP_REQUIRE(oy >= 0 && ox >= 0 && ox + W <= pos_w && oy + H <= pos_h,
+                "positional-encoding crop [%d:%d,%d:%d] outside the %dx%d table", oy, oy + H, ox, ox + W, pos_h, pos_w);
+    return posenc_tokens_nhwc_f32(x, x_pitch, pos, tokens, B, C, H, W, pos_w, oy, ox, (cudaStream_t)stream);
+}
+CFP_API int cfp_copy_channels_f32(const float* src, int src_pitch, float* dst, int dst_pitch, int coff, int C, int64_t rows, void* stream) {
+    begin_call(stream);
+    CFP_REQUIRE(src && dst && rows >= 0, "bad arguments");
+    return copy_channels_f32(src, src_pitch, dst, dst_pitch, coff, C, rows, (cudaStream_t)stream);
+}
+CFP_API int cfp_head_bins_f32(const float* x, int pitch, int B, int npix, int E, const float* wc, const float* w0, const float* b0,
+                              const float* w2, const float* b2, const float* w4, const float* b4, int hidden, int n_bins, float min_val,
+                              float max_val, float* mean_scratch, float* edges, float* centres, void* stream) {
+    begin_call(stream);
+    CFP_REQUIRE(x && wc && w0 && b0 && w2 && b2 && w4 && b4 && mean_scratch && edges && centres, "null pointer");
+    if (int e = channel_mean_f32(x, pitch, E, B, npix, mean_scratch, (cudaStream_t)stream)) return e;
+    return head_regressor(mean_scratch, wc, w0, b0, w2, b2, w4, b4, B, E, hidden, n_bins, min_val, max_val, edges, centres,
+                          (cudaStream_t)stream);
+}
+CFP_API int cfp_head_expect_f32(const float* x, int pitch, int B, int npix, const float* w_t, const float* bias, const float* centres,
+                                int n_bins, float* pred, float* prob, void* stream) {
+    begin_call(stream);
+    CFP_REQUIRE(x && w_t && bias && centres && pred, "null pointer");
+    return head_expect_f32(x, pitch, B, npix, w_t, bias, centres, n_bins, pred, prob, (cudaStream_t)stream);
+}
+
 CFP_API int cfp_selftest_umma(const void* a, const void* b, float* d, int rows_a, int n, int k, int row_shift,
                               void* stream) {
     begin_call(stream);

@@ -129,6 +129,18 @@ int head_regressor(const float* mean, const float* wc, const float* w0, const fl
 int head_expect_tc(const void* x, int pitch, int B, int npix, const void* w_tc, const float* bias, const float* centres, int nb, float* pred,
                    float* prob, cudaStream_t st);
 
+// k_dec_f32.cu  (decoder shell f1, adaptive-bins head f2; exact fp32 engine, channels-last)
+int conv_f32(const float* in, int cin, int taps, const float* w, const float* shift, float slope, float* out, int out_pitch, int out_coff,
+             int B, int H, int W, int cout, cudaStream_t st);
+int upsample_concat_f32(const float* lo, int h, int w, int c_lo, int lo_pitch, const float* skip, int c_skip, float* out, int B, int H, int W,
+                        int c_out, cudaStream_t st);
+int copy_channels_f32(const float* src, int src_pitch, float* dst, int dst_pitch, int coff, int C, int64_t rows, cudaStream_t st);
+int posenc_tokens_nhwc_f32(const float* x, int x_pitch, const float* pos, float* tokens, int B, int C, int H, int W, int pos_w, int oy, int ox,
+                           cudaStream_t st);
+int channel_mean_f32(const float* x, int pitch, int C, int B, int npix, float* mean, cudaStream_t st);
+int head_expect_f32(const float* x, int pitch, int B, int npix, const float* w_t, const float* bias, const float* centres, int nb, float* pred,
+                    float* prob, cudaStream_t st);
+
 // k_selftest.cu
 int umma_selftest(const void* A, const void* B, float* D, int rows_a, int N, int K, int row_shift, cudaStream_t st);
 

@@ -121,16 +121,18 @@ class TransformerFusion(nn.Module):
         return False
 
     def forward_tokens(self, x_tok, x_pitch, B, H, W, feat1, out_tok, out_pitch, out_coff, **kwargs):
-        """The same call for a caller that holds its maps channels-last in bf16 (cfpnet_b200.decoder): ``x_tok`` is a
+        """The same call for a caller that holds its maps channels-last (cfpnet_b200.decoder): ``x_tok`` is a
         [B, H, W, x_pitch] buffer whose first ``embedding_dim`` channels are x; the result is written into channels
         [out_coff, out_coff + embedding_dim) of ``out_tok`` [B, H, W, out_pitch] - the ``torch.cat([x_d, x_d_fused])`` of
-        decoder.py:112,117,122 without a transposed or concatenated copy.  Same positional-encoding draws as forward()."""
+        decoder.py:112,117,122 without a transposed or concatenated copy.  Same positional-encoding draws as forward().
+        Both maps bf16 run the tensor-core engine, both fp32 the exact fp32 engine (the module's parameters in fp32)."""
         if self.training:
             raise NotImplementedError("libcfp serves eval-mode BatchNorm only for the attention layers")
         _lib.require_cuda(x_tok, "x_tok")
         D = self.embedding_dim
-        if x_tok.dtype != torch.bfloat16 or out_tok.dtype != torch.bfloat16:
-            raise ValueError("forward_tokens serves the bf16 engine")
+        dt = x_tok.dtype
+        if dt not in (torch.bfloat16, torch.float32) or out_tok.dtype != dt:
+            raise ValueError(f"forward_tokens needs x_tok and out_tok both bf16 or both fp32 (got {x_tok.dtype} and {out_tok.dtype})")
         S = feat1.size(2)
         g = zone_geometry(kwargs["patch_info"], self.max_resolution[1], H, W)
         if any(n in ("hist2image", "combine1") for n in self.layer_names):
@@ -144,8 +146,9 @@ class TransformerFusion(nn.Module):
         oy, ox = self.draw_crop(H, W)
         packed, pos, pos2, _buf = self._cache.get(self, self._pack)
         dev = x_tok.device
-        dt = torch.bfloat16
-        code = _lib.CFP_BF16
+        code = _lib.dtype_code(dt)
+        posenc, copy = (("cfp_posenc_tokens_nhwc_f32_fwd", "cfp_copy_channels_f32") if dt == torch.float32
+                        else ("cfp_posenc_tokens_nhwc_fwd", "cfp_copy_channels"))
         feat1 = feat1.detach().to(dt).contiguous()
         mask = kwargs["mask"].to(device=dev, dtype=torch.uint8).contiguous()
         cg = _lib.CfpGeom.from_geometry(g)
@@ -157,10 +160,10 @@ class TransformerFusion(nn.Module):
                 dev.index, (dt, B, H, W), lambda t: t[0].numel() >= ws_bytes,
                 lambda: (torch.empty(ws_bytes, device=dev, dtype=torch.uint8), torch.empty(B, H * W, D, device=dev, dtype=dt)))
             st = _lib.stream_ptr()
-            _lib.call("cfp_posenc_tokens_nhwc_fwd", x_tok.data_ptr(), x_pitch, pos, feat0.data_ptr(), B, D, H, W,
+            _lib.call(posenc, x_tok.data_ptr(), x_pitch, pos, feat0.data_ptr(), B, D, H, W,
                       self.max_resolution[0], self.max_resolution[1], oy, ox, st)
             self._run_layers(packed, pos2, feat0, feat1, mask, B, H, W, D, S, cg, work, ws_bytes, code, st, emb_copy)
-            _lib.call("cfp_copy_channels", feat0.data_ptr(), D, out_tok.data_ptr(), out_pitch, out_coff, D, B * H * W, st)
+            _lib.call(copy, feat0.data_ptr(), D, out_tok.data_ptr(), out_pitch, out_coff, D, B * H * W, st)
         return out_tok
 
     # ------------------------------------------------------------------ forward

@@ -318,6 +318,31 @@ CFP_API int cfp_head_bins(const void *x, int pitch, int B, int npix, int E, cons
 CFP_API int cfp_head_expect(const void *x, int pitch, int B, int npix, const void *w_tc, const float *bias, const float *centres,
                             int n_bins, float *pred, float *prob, void *stream);
 
+/* ---- The same stages on the exact fp32 engine: fp32 channels-last maps, fp32 FFMA with fp32 accumulation (no TF32 or bf16
+ * operands), no atomics (every output is summed in one fixed order: two runs give the same bits).  Each call has the
+ * contract of its bf16 sibling above, except:
+ * cfp_conv_f32_fwd: cin is a multiple of 4 and equal to the input's pitch (no padding, no K-chunk argument); w is fp32
+ *   [k * k][cin][cout] (tap = ky * k + kx); out_pitch and out_coff are multiples of 4.
+ * cfp_upsample_concat_f32, cfp_copy_channels_f32, cfp_posenc_tokens_nhwc_f32_fwd: channel counts, pitches and offsets are
+ *   multiples of 4.
+ * cfp_head_bins_f32: x is fp32; the channel mean is formed per frame in one CTA (no atomics), then the regressor of
+ *   cfp_head_bins.
+ * cfp_head_expect_f32: x fp32 [B][npix][pitch]; w_t = conv_out's weight as fp32 [128][n_bins]; softmax with expf and true
+ *   divisions. */
+CFP_API int cfp_conv_f32_fwd(const float *in, int B, int H, int W, int cin, int cout, int ksize, const float *w, const float *shift,
+                             float leaky_slope, float *out, int out_pitch, int out_coff, void *stream);
+CFP_API int cfp_upsample_concat_f32(const float *lo, int h, int w, int c_lo, int lo_pitch, const float *skip, int c_skip, float *out,
+                                    int B, int H, int W, int c_out, void *stream);
+CFP_API int cfp_posenc_tokens_nhwc_f32_fwd(const float *x, int x_pitch, const float *pos, float *tokens, int B, int C, int H, int W,
+                                           int pos_h, int pos_w, int oy, int ox, void *stream);
+CFP_API int cfp_copy_channels_f32(const float *src, int src_pitch, float *dst, int dst_pitch, int coff, int C, int64_t rows,
+                                  void *stream);
+CFP_API int cfp_head_bins_f32(const float *x, int pitch, int B, int npix, int E, const float *wc, const float *w0, const float *b0,
+                              const float *w2, const float *b2, const float *w4, const float *b4, int hidden, int n_bins,
+                              float min_val, float max_val, float *mean_scratch, float *edges, float *centres, void *stream);
+CFP_API int cfp_head_expect_f32(const float *x, int pitch, int B, int npix, const float *w_t, const float *bias, const float *centres,
+                                int n_bins, float *pred, float *prob, void *stream);
+
 /* ---- Input side (SURVEY.md 8 f3; the reference runs these on the host CPU inside its dataloader, one frame at a time).
  *
  * cfp_zone_hist: get_hist_parallel (src/utils/dataloader.py:84-134) for a batch of depth maps dep [B][H][W] (metres):
