@@ -104,6 +104,11 @@ SIGNATURES = {
     "cfp_copy_channels_f32": (_i, [_p, _i, _p, _i, _i, _i, _i64, _p]),
     "cfp_head_bins_f32": (_i, [_p, _i, _i, _i, _i] + [_p] * 7 + [_i, _i, C.c_float, C.c_float, _p, _p, _p, _p]),
     "cfp_head_expect_f32": (_i, [_p, _i, _i, _i, _p, _p, _p, _i, _p, _p, _p]),
+    "cfp_tr_conv_wgrad_scratch_floats": (_sz, [_i] * 6),
+    "cfp_tr_conv_wgrad_f32": (_i, [_p, _p, _p, _p] + [_i] * 6 + [_p]),
+    "cfp_tr_upsample_concat_bwd_f32": (_i, [_p, _i, _p, _i, _i, _i, _p, _i, _i, _i, _i, _p]),
+    "cfp_tr_head_expect_bwd_f32": (_i, [_p, _p, _p, _p, _i, _i, _i, _p, _p, _p, _p]),
+    "cfp_tr_head_bins_bwd_f32": (_i, [_p, _p, _p, _p, _i, _i, C.c_float, C.c_float, _p]),
     "cfp_zone_hist": (_i, [_p] + [_i] * 9 + [C.c_float, _p, _p, _p, _p, _p]),
     "cfp_zone_samples": (_i, [_p, _p, _p, _i64, _i, _p, _p, _i, _p]),
     "cfp_silog_fwd": (_i, [_p, _p, _p] + [_i] * 6 + [_p, _p, _p]),

@@ -594,6 +594,36 @@ CFP_API int cfp_head_expect_f32(const float* x, int pitch, int B, int npix, cons
     return head_expect_f32(x, pitch, B, npix, w_t, bias, centres, n_bins, pred, prob, (cudaStream_t)stream);
 }
 
+// the decoder shell and head in train mode (k_dec_train.cu)
+CFP_API size_t cfp_tr_conv_wgrad_scratch_floats(int B, int H, int W, int cin, int cout, int ksize) {
+    return (ksize == 1 || ksize == 3) ? conv_wgrad_scratch_floats(B, H, W, cin, cout, ksize * ksize) : 0;
+}
+CFP_API int cfp_tr_conv_wgrad_f32(const float* x, const float* dy, float* dw, float* scratch, int B, int H, int W, int cin, int cout,
+                                  int ksize, void* stream) {
+    begin_call(stream);
+    CFP_REQUIRE(x && dy && dw, "null pointer");
+    CFP_REQUIRE(ksize == 1 || ksize == 3, "kernel size %d (1 and 3 are served)", ksize);
+    return conv_wgrad_f32(x, dy, dw, scratch, B, H, W, cin, cout, ksize * ksize, (cudaStream_t)stream);
+}
+CFP_API int cfp_tr_upsample_concat_bwd_f32(const float* dcat, int pitch, float* d_lo, int h, int w, int c_lo, float* d_skip, int c_skip,
+                                           int B, int H, int W, void* stream) {
+    begin_call(stream);
+    CFP_REQUIRE(dcat, "null pointer");
+    return upsample_concat_bwd_f32(dcat, pitch, d_lo, h, w, c_lo, d_skip, c_skip, B, H, W, (cudaStream_t)stream);
+}
+CFP_API int cfp_tr_head_expect_bwd_f32(const float* prob, const float* pred, const float* centres, const float* dpred, int B, int npix,
+                                       int n_bins, float* dlogit, float* dcentres, float* scratch, void* stream) {
+    begin_call(stream);
+    CFP_REQUIRE(prob && pred && centres && dpred && dlogit && dcentres && scratch, "null pointer");
+    return head_expect_bwd_f32(prob, pred, centres, dpred, B, npix, n_bins, dlogit, dcentres, scratch, (cudaStream_t)stream);
+}
+CFP_API int cfp_tr_head_bins_bwd_f32(const float* z, const float* d_edges, const float* d_centres, float* dz, int B, int n_bins,
+                                     float min_val, float max_val, void* stream) {
+    begin_call(stream);
+    CFP_REQUIRE(z && dz, "null pointer");
+    return head_bins_bwd_f32(z, d_edges, d_centres, dz, B, n_bins, min_val, max_val, (cudaStream_t)stream);
+}
+
 CFP_API int cfp_selftest_umma(const void* a, const void* b, float* d, int rows_a, int n, int k, int row_shift,
                               void* stream) {
     begin_call(stream);

@@ -141,6 +141,17 @@ int channel_mean_f32(const float* x, int pitch, int C, int B, int npix, float* m
 int head_expect_f32(const float* x, int pitch, int B, int npix, const float* w_t, const float* bias, const float* centres, int nb, float* pred,
                     float* prob, cudaStream_t st);
 
+// k_dec_train.cu  (decoder shell and head in train mode: the adjoints with no forward counterpart; fp32, channels-last)
+size_t conv_wgrad_scratch_floats(int B, int H, int W, int cin, int cout, int taps);
+int conv_wgrad_f32(const float* x, const float* dy, float* dw, float* scratch, int B, int H, int W, int cin, int cout, int taps,
+                   cudaStream_t st);
+int upsample_concat_bwd_f32(const float* dcat, int pitch, float* d_lo, int h, int w, int c_lo, float* d_skip, int c_skip, int B, int H, int W,
+                            cudaStream_t st);
+int head_expect_bwd_f32(const float* prob, const float* pred, const float* centres, const float* dpred, int B, int npix, int nb, float* dlogit,
+                        float* dcentres, float* scratch, cudaStream_t st);
+int head_bins_bwd_f32(const float* z, const float* d_edges, const float* d_centres, float* dz, int B, int nb, float min_val, float max_val,
+                      cudaStream_t st);
+
 // k_selftest.cu
 int umma_selftest(const void* A, const void* B, float* D, int rows_a, int N, int K, int row_shift, cudaStream_t st);
 

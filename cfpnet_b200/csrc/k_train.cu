@@ -363,6 +363,7 @@ int tr_ln_bwd(const float* x, const float* g, const float* dy, float* dx, float*
 // op 2: out = gelu_erf(a)      op 3: out = a * gelu_erf'(b)   (convnext.py:33: nn.GELU(), erf form)
 // op 4: out = relu(a)          op 5: out = a * elu1'(b) = a * (b > 0 ? 1 : exp(b))
 // op 6: out = elu(a) + 1       op 7: out = -a / b             (attention.py:10-11; the normaliser's gradient)
+// op 8: out = leaky_relu(a)    op 9: out = a * (b > 0 ? 1 : 0.01)  (nn.LeakyReLU() of decoder.py, slope 0.01)
 __global__ void __launch_bounds__(256) tr_ew_kernel(const float* __restrict__ a, const float* __restrict__ b, float* __restrict__ out,
                                                     int64_t n, int op) {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
@@ -380,14 +381,16 @@ __global__ void __launch_bounds__(256) tr_ew_kernel(const float* __restrict__ a,
             case 4: r = fmaxf(x, 0.f); break;
             case 6: r = x > 0.f ? x + 1.f : expf(x); break;
             case 7: r = -x / b[i]; break;
+            case 8: r = x > 0.f ? x : 0.01f * x; break;
+            case 9: r = b[i] > 0.f ? x : 0.01f * x; break;
             default: { const float t = b[i]; r = t > 0.f ? x : x * __expf(t); break; }
         }
         out[i] = r;
     }
 }
 int tr_ew(const float* a, const float* b, float* out, int64_t n, int op, cudaStream_t st) {
-    CFP_REQUIRE(op >= 0 && op <= 7, "tr_ew: unknown op %d", op);
-    CFP_REQUIRE(b != nullptr || op == 2 || op == 4 || op == 6, "tr_ew: op %d needs a second operand", op);
+    CFP_REQUIRE(op >= 0 && op <= 9, "tr_ew: unknown op %d", op);
+    CFP_REQUIRE(b != nullptr || op == 2 || op == 4 || op == 6 || op == 8, "tr_ew: op %d needs a second operand", op);
     if (n == 0) return 0;
     tr_ew_kernel<<<ew_grid(n), 256, 0, st>>>(a, b, out, n, op);
     return check_launch("tr_ew");

@@ -8,7 +8,8 @@ the fusion layers): every ``torch.cat`` of the reference is a write into a slice
 upsample + skip concat is one kernel, convs are ``cfp_conv_fwd`` (tcgen05 implicit GEMM with the eval-mode BatchNorm folded
 and LeakyReLU in the epilogue), and ``conv_out`` + softmax + bin expectation is ``cfp_head_expect`` (the 256-bin
 probability volume is only written on request).  The fp32 engine runs the same sequence on fp32 maps through
-the ``*_f32`` kernels (FFMA, fixed summation order) and the fusion modules' fp32 engine.  Eval mode only; no CPU fallback.
+the ``*_f32`` kernels (FFMA, fixed summation order) and the fusion modules' fp32 engine.  In ``.train()`` mode ``forward``
+runs the fp32 training path of cfpnet_b200/decoder_train.py.  No CPU fallback.
 """
 from __future__ import annotations
 
@@ -102,9 +103,14 @@ class Decoder(nn.Module):
     """decoder.py:60-128.  ``forward(img_features, hist_features, **kwargs)`` returns the reference's ``[B, num_classes,
     h/2, w/2]`` map (NCHW, fp32); ``forward_nhwc`` returns it channels-last in ``compute_dtype`` for ``DepthHead``.
 
-    ``compute_dtype`` selects the engine: ``torch.bfloat16`` (default) runs the tcgen05 kernels with bf16 maps and the
-    fusion modules in whatever dtype they were cast to (bf16 for the tensor-core engine); ``torch.float32`` runs the
-    exact fp32 kernels on fp32 maps and needs the ``cross_atten*`` modules left in fp32 (their fp32 engine)."""
+    ``compute_dtype`` selects the eval engine: ``torch.bfloat16`` (default) runs the tcgen05 kernels with bf16 maps and
+    the fusion modules in whatever dtype they were cast to (bf16 for the tensor-core engine); ``torch.float32`` runs the
+    exact fp32 kernels on fp32 maps and needs the ``cross_atten*`` modules left in fp32 (their fp32 engine).
+
+    In ``.train()`` mode ``forward`` runs the fp32 training path (cfpnet_b200/decoder_train.py) and does not consult
+    ``compute_dtype``: BatchNorm on batch statistics (running buffers updated), the ``cross_atten*`` modules through their
+    train path, and the map differentiable w.r.t. every parameter, the five ``img_features`` and ``hist_features``.
+    Parameters and inputs must be fp32 CUDA tensors (``CfpError`` otherwise)."""
 
     LEAKY = 0.01                                  # nn.LeakyReLU() default
 
@@ -220,6 +226,9 @@ class Decoder(nn.Module):
         return out, H0, W0
 
     def forward(self, img_features, hist_features, **kwargs):
+        if self.training:
+            from .decoder_train import decoder_train_forward
+            return decoder_train_forward(self, img_features, hist_features, **kwargs)
         out, H, W = self.forward_nhwc(img_features, hist_features, **kwargs)
         B = out.shape[0]
         res = torch.empty(B, self.num_classes, H, W, device=out.device, dtype=out.dtype)
@@ -247,8 +256,11 @@ class DepthRegression(nn.Module):
 
 class DepthHead(nn.Module):
     """The part of ``Deltar`` below the decoder (deltar.py:16-19, 50-61): ``depth_head`` + ``conv_out`` -> (bin_edges
-    [B, n_bins + 1], pred [B, 1, H, W][, prob [B, n_bins, H, W]]).  Consumes the decoder's channels-last map: a bf16 map
-    runs the tcgen05 head, an fp32 map the exact fp32 one."""
+    [B, n_bins + 1], pred [B, 1, H, W][, prob [B, n_bins, H, W]]).  ``forward_nhwc`` consumes the decoder's channels-last
+    map: a bf16 map runs the tcgen05 head, an fp32 map the exact fp32 one.  ``forward(unet_out)`` takes the NCHW map
+    ``Decoder.forward`` returns (deltar.py:50-61): in eval mode it flips the layout and runs ``forward_nhwc`` (the engine
+    follows the map's dtype); in ``.train()`` mode it runs the fp32 training path (cfpnet_b200/decoder_train.py),
+    differentiable w.r.t. the map and every head parameter."""
 
     def __init__(self, n_bins=256, min_val=1e-3, max_val=10.0, norm="linear"):
         super().__init__()
@@ -302,3 +314,18 @@ class DepthHead(nn.Module):
             _lib.call(expect, ram.data_ptr(), 128, B, H * W, P["wout"].data_ptr(), P["bout"].data_ptr(), centres.data_ptr(),
                       nb, pred.data_ptr(), _lib.ptr(prob), st)
         return (edges, pred, prob) if return_prob else (edges, pred)
+
+    def forward(self, unet_out: torch.Tensor):
+        if self.training:
+            from .decoder_train import head_train_forward
+            return head_train_forward(self, unet_out)
+        _lib.require_cuda(unet_out, "unet_out")
+        B, E, H, W = unet_out.shape
+        dt = unet_out.dtype
+        if dt not in (torch.bfloat16, torch.float32):
+            raise ValueError(f"unet_out must be bfloat16 (tensor-core head) or float32 (exact fp32 head), not {dt}")
+        x = torch.empty(B, H, W, E, device=unet_out.device, dtype=dt)
+        with torch.cuda.device(unet_out.device):
+            _lib.call("cfp_upsample_concat_f32" if dt == torch.float32 else "cfp_upsample_concat", 0, 1, 1, 0, 8,
+                      unet_out.detach().float().contiguous().data_ptr(), E, x.data_ptr(), B, H, W, E, _lib.stream_ptr())
+        return self.forward_nhwc(x, H, W)

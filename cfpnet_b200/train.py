@@ -20,6 +20,7 @@ from typing import Dict, List, Tuple
 import torch
 
 from . import _lib
+from .packing import PackCache
 
 BN_EPS, BN_MOMENTUM = 1e-5, 0.1          # nn.BatchNorm defaults (encoder.py:10-12, convnext.py:39, transformer.py:198-200)
 LKPM_LN_EPS = 1e-6                       # convnext.py:31
@@ -581,8 +582,8 @@ class FlatTrainer:
                       self.flat_v.data_ptr(), n, self.seg_end.data_ptr(), self.seg_lr.data_ptr(), int(self.seg_lr.numel()),
                       C.c_float(self.betas[0]), C.c_float(self.betas[1]), C.c_float(self.eps), C.c_float(self.wd),
                       self.step_count, C.c_float(scale), self.sumsq.data_ptr(), C.c_float(self.max_norm), _st())
-        for m in self.modules:               # packed eval-mode weights of the modules are stale now
+        for m in self.modules:               # packed eval-mode weights of the modules are stale now (every engine's cache)
             for sub in m.modules():
-                cache = getattr(sub, "_cache", None)
-                if cache is not None and hasattr(cache, "invalidate"):
-                    cache.invalidate()
+                for cache in list(vars(sub).values()):
+                    if isinstance(cache, PackCache):
+                        cache.invalidate()

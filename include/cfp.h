@@ -231,7 +231,8 @@ CFP_API int cfp_tr_ln_fwd(const float *x, const float *g, const float *b, float 
 CFP_API int cfp_tr_ln_bwd(const float *x, const float *g, const float *dy, float *dx, float *dg, float *db, int64_t rows,
                           int C, float eps, void *stream);
 /* Elementwise: op 0 out = a + b | 1 out = a * (b > 0) | 2 out = gelu_erf(a) | 3 out = a * gelu_erf'(b) | 4 out = relu(a)
- * | 5 out = a * d/db(elu(b) + 1) | 6 out = elu(a) + 1 | 7 out = -a / b. */
+ * | 5 out = a * d/db(elu(b) + 1) | 6 out = elu(a) + 1 | 7 out = -a / b | 8 out = leaky_relu(a, 0.01) (nn.LeakyReLU() of
+ * decoder.py) | 9 out = a * (b > 0 ? 1 : 0.01), its gradient. */
 CFP_API int cfp_tr_ew(const float *a, const float *b, float *out, int64_t n, int op, void *stream);
 /* ---- second slice of the training step: the linear-attention layers and the DAPM convolutions of a TransformerFusion
  * call in train mode (fusion.py:52-188, transformer.py:41-71,89-150,204-248, attention.py:31-49 under autograd in the
@@ -342,6 +343,34 @@ CFP_API int cfp_head_bins_f32(const float *x, int pitch, int B, int npix, int E,
                               float min_val, float max_val, float *mean_scratch, float *edges, float *centres, void *stream);
 CFP_API int cfp_head_expect_f32(const float *x, int pitch, int B, int npix, const float *w_t, const float *bias, const float *centres,
                                 int n_bins, float *pred, float *prob, void *stream);
+
+/* ---- The decoder shell and head in train mode (reference train.py:96-135 differentiates decoder.py / deltar.py:50-61 with
+ * autograd): the adjoints no forward kernel computes.  fp32 FFMA, no atomics, fixed summation order (two launches give the
+ * same bits).  cfpnet_b200/decoder_train.py sequences them with the forward kernels above: a conv's input gradient is
+ * cfp_conv_f32_fwd with the taps mirrored and in / out channels swapped.
+ *
+ * cfp_tr_conv_wgrad_f32: weight gradient of a k x k conv (k = 1, 3; stride 1, zero padding k / 2) on channels-last maps,
+ *   dw[tap][ci][co] = sum_{b,y,x} x[b][y + ky - k/2][x + kx - k/2][ci] dy[b][y][x][co] (tap = ky k + kx: the fp32 weight
+ *   layout of cfp_conv_f32_fwd).  cin, cout multiples of 4; x has pitch cin, dy pitch cout.  The B*H*W pixels are split
+ *   into ranges, each writes a partial into `scratch`, a second pass adds them in range order:
+ *   cfp_tr_conv_wgrad_scratch_floats(B, H, W, cin, cout, ksize) floats (pure host arithmetic; 0 = no scratch needed).
+ * cfp_tr_upsample_concat_bwd_f32: adjoint of cfp_upsample_concat_f32.  dcat [B][H][W][pitch] -> d_lo [B][h][w][c_lo]
+ *   (channels-last, the adjoint of the align_corners bilinear resize, gathered per low-resolution pixel) and d_skip
+ *   [B][c_skip][H][W] (NCHW, channels c_lo .. c_lo + c_skip of dcat).
+ * cfp_tr_head_expect_bwd_f32: adjoint of cfp_head_expect_f32 given its probability volume prob [B][n_bins][npix], pred
+ *   [B][npix], centres [B][n_bins] and dpred [B][npix]: dlogit [B*npix][n_bins] = p (centre - pred) dpred, dcentres
+ *   [B][n_bins] = sum_pixels p dpred.  scratch: B * ((npix + 31) / 32) * n_bins floats.
+ * cfp_tr_head_bins_bwd_f32: one CTA per frame.  z [B][n_bins] = the regressor's output before relu + 0.1; d_edges [B][n_bins
+ *   + 1] and d_centres [B][n_bins] (either nullable = zero) are the cotangents of cfp_head_bins_f32's outputs -> dz. */
+CFP_API size_t cfp_tr_conv_wgrad_scratch_floats(int B, int H, int W, int cin, int cout, int ksize);
+CFP_API int cfp_tr_conv_wgrad_f32(const float *x, const float *dy, float *dw, float *scratch, int B, int H, int W, int cin, int cout,
+                                  int ksize, void *stream);
+CFP_API int cfp_tr_upsample_concat_bwd_f32(const float *dcat, int pitch, float *d_lo, int h, int w, int c_lo, float *d_skip, int c_skip,
+                                           int B, int H, int W, void *stream);
+CFP_API int cfp_tr_head_expect_bwd_f32(const float *prob, const float *pred, const float *centres, const float *dpred, int B, int npix,
+                                       int n_bins, float *dlogit, float *dcentres, float *scratch, void *stream);
+CFP_API int cfp_tr_head_bins_bwd_f32(const float *z, const float *d_edges, const float *d_centres, float *dz, int B, int n_bins,
+                                     float min_val, float max_val, void *stream);
 
 /* ---- Input side (SURVEY.md 8 f3; the reference runs these on the host CPU inside its dataloader, one frame at a time).
  *
