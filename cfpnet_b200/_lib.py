@@ -95,12 +95,14 @@ SIGNATURES = {
     "cfp_upsample_concat": (_i, [_p, _i, _i, _i, _i, _p, _i, _p, _i, _i, _i, _i, _p]),
     "cfp_posenc_tokens_crop_fwd": (_i, [_p, _p, _p] + [_i] * 6 + [_p, _i, _p]),
     "cfp_posenc_tokens_nhwc_fwd": (_i, [_p, _i, _p, _p] + [_i] * 8 + [_p]),
+    "cfp_posenc_tokens_nhwc_crop_fwd": (_i, [_p, _i, _p, _p] + [_i] * 6 + [_p, _p]),
     "cfp_copy_channels": (_i, [_p, _i, _p, _i, _i, _i, _i64, _p]),
     "cfp_head_bins": (_i, [_p, _i, _i, _i, _i] + [_p] * 7 + [_i, _i, C.c_float, C.c_float, _p, _p, _p, _p]),
     "cfp_head_expect": (_i, [_p, _i, _i, _i, _p, _p, _p, _i, _p, _p, _p]),
     "cfp_conv_f32_fwd": (_i, [_p] + [_i] * 6 + [_p, _p, C.c_float, _p, _i, _i, _p]),
     "cfp_upsample_concat_f32": (_i, [_p, _i, _i, _i, _i, _p, _i, _p, _i, _i, _i, _i, _p]),
     "cfp_posenc_tokens_nhwc_f32_fwd": (_i, [_p, _i, _p, _p] + [_i] * 8 + [_p]),
+    "cfp_posenc_tokens_nhwc_f32_crop_fwd": (_i, [_p, _i, _p, _p] + [_i] * 6 + [_p, _p]),
     "cfp_copy_channels_f32": (_i, [_p, _i, _p, _i, _i, _i, _i64, _p]),
     "cfp_head_bins_f32": (_i, [_p, _i, _i, _i, _i] + [_p] * 7 + [_i, _i, C.c_float, C.c_float, _p, _p, _p, _p]),
     "cfp_head_expect_f32": (_i, [_p, _i, _i, _i, _p, _p, _p, _i, _p, _p, _p]),

@@ -529,6 +529,14 @@ CFP_API int cfp_posenc_tokens_nhwc_fwd(const void* x, int x_pitch, const float* 
                 "positional-encoding crop [%d:%d,%d:%d] outside the %dx%d table", oy, oy + H, ox, ox + W, pos_h, pos_w);
     return posenc_tokens_nhwc(x, x_pitch, pos, tokens, B, C, H, W, pos_w, oy, ox, (cudaStream_t)stream);
 }
+CFP_API int cfp_posenc_tokens_nhwc_crop_fwd(const void* x, int x_pitch, const float* pos, void* tokens, int B, int C, int H, int W,
+                                            int pos_h, int pos_w, const int* crop, void* stream) {
+    begin_call(stream);
+    CFP_REQUIRE(x && pos && tokens && crop, "null pointer");
+    CFP_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, "bad shape");
+    CFP_REQUIRE(W <= pos_w && H <= pos_h, "feature map %dx%d larger than the %dx%d positional-encoding table", H, W, pos_h, pos_w);
+    return posenc_tokens_nhwc(x, x_pitch, pos, tokens, B, C, H, W, pos_w, 0, 0, (cudaStream_t)stream, crop);
+}
 CFP_API int cfp_copy_channels(const void* src, int src_pitch, void* dst, int dst_pitch, int coff, int C, int64_t rows, void* stream) {
     begin_call(stream);
     CFP_REQUIRE(src && dst && rows >= 0, "bad arguments");
@@ -572,6 +580,14 @@ CFP_API int cfp_posenc_tokens_nhwc_f32_fwd(const float* x, int x_pitch, const fl
     CFP_REQUIRE(oy >= 0 && ox >= 0 && ox + W <= pos_w && oy + H <= pos_h,
                 "positional-encoding crop [%d:%d,%d:%d] outside the %dx%d table", oy, oy + H, ox, ox + W, pos_h, pos_w);
     return posenc_tokens_nhwc_f32(x, x_pitch, pos, tokens, B, C, H, W, pos_w, oy, ox, (cudaStream_t)stream);
+}
+CFP_API int cfp_posenc_tokens_nhwc_f32_crop_fwd(const float* x, int x_pitch, const float* pos, float* tokens, int B, int C, int H,
+                                                int W, int pos_h, int pos_w, const int* crop, void* stream) {
+    begin_call(stream);
+    CFP_REQUIRE(x && pos && tokens && crop, "null pointer");
+    CFP_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, "bad shape");
+    CFP_REQUIRE(W <= pos_w && H <= pos_h, "feature map %dx%d larger than the %dx%d positional-encoding table", H, W, pos_h, pos_w);
+    return posenc_tokens_nhwc_f32(x, x_pitch, pos, tokens, B, C, H, W, pos_w, 0, 0, (cudaStream_t)stream, crop);
 }
 CFP_API int cfp_copy_channels_f32(const float* src, int src_pitch, float* dst, int dst_pitch, int coff, int C, int64_t rows, void* stream) {
     begin_call(stream);

@@ -242,9 +242,12 @@ int copy_channels_f32(const float* src, int src_pitch, float* dst, int dst_pitch
     return check_launch("copy_channels_f32");
 }
 
+// kCropDev: (oy, ox) from device memory, as posenc_tokens_nhwc_kernel (k_dec_tc.cu)
+template <bool kCropDev>
 __global__ void __launch_bounds__(256) posenc_tokens_nhwc_f32_kernel(const float* __restrict__ x, int x_pitch, const float* __restrict__ pos,
                                                                      float* __restrict__ tokens, int B, int C, int H, int W, int pos_w,
-                                                                     int oy, int ox) {
+                                                                     int oy, int ox, const int* __restrict__ crop) {
+    if (kCropDev) { oy = crop[0]; ox = crop[1]; }
     const int groups = C / 4;
     const int64_t total = (int64_t)B * H * W * groups;
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
@@ -257,10 +260,14 @@ __global__ void __launch_bounds__(256) posenc_tokens_nhwc_f32_kernel(const float
     }
 }
 int posenc_tokens_nhwc_f32(const float* x, int x_pitch, const float* pos, float* tokens, int B, int C, int H, int W, int pos_w, int oy, int ox,
-                           cudaStream_t st) {
+                           cudaStream_t st, const int* crop) {
     CFP_REQUIRE(C % 4 == 0 && x_pitch % 4 == 0 && C <= x_pitch, "posenc_tokens_nhwc_f32: C = %d, pitch %d", C, x_pitch);
-    posenc_tokens_nhwc_f32_kernel<<<grid_for((int64_t)B * H * W * (C / 4)), 256, 0, st>>>(x, x_pitch, pos, tokens, B, C, H, W, pos_w, oy,
-                                                                                          ox);
+    const auto grid = grid_for((int64_t)B * H * W * (C / 4));
+    if (crop) {
+        posenc_tokens_nhwc_f32_kernel<true><<<grid, 256, 0, st>>>(x, x_pitch, pos, tokens, B, C, H, W, pos_w, 0, 0, crop);
+        return check_launch("posenc_tokens_nhwc_f32_crop");
+    }
+    posenc_tokens_nhwc_f32_kernel<false><<<grid, 256, 0, st>>>(x, x_pitch, pos, tokens, B, C, H, W, pos_w, oy, ox, nullptr);
     return check_launch("posenc_tokens_nhwc_f32");
 }
 

@@ -323,11 +323,15 @@ int copy_channels(const void* src, int src_pitch, void* dst, int dst_pitch, int 
 
 // ------------------------------------------------------------------------------------------------ pos-enc add on a channels-last map
 // tokens[b][n][:] = x[b][n][0 : C] (pitch x_pitch) + pos[(oy + y) * pos_w + ox + x][:]   (fusion.py:87-97 for a caller that already
-// holds the map channels-last: the decoder shell above - no NCHW round trip between the convs and the fusion layers)
+// holds the map channels-last: the decoder shell above - no NCHW round trip between the convs and the fusion layers).
+// kCropDev: (oy, ox) = crop[0], crop[1], read from device memory when the kernel runs (a CUDA-graph replay takes fresh draws);
+// otherwise the by-value offsets, and `crop` is not read.
+template <bool kCropDev>
 __global__ void __launch_bounds__(256) posenc_tokens_nhwc_kernel(const bf16* __restrict__ x, int x_pitch, const float* __restrict__ pos,
                                                                  bf16* __restrict__ tokens, int B, int C, int H, int W, int pos_w, int oy,
-                                                                 int ox) {
+                                                                 int ox, const int* __restrict__ crop) {
     pdl_wait();
+    if (kCropDev) { oy = crop[0]; ox = crop[1]; }
     const int groups = C / 8;
     const int64_t total = (int64_t)B * H * W * groups;
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
@@ -347,12 +351,18 @@ __global__ void __launch_bounds__(256) posenc_tokens_nhwc_kernel(const bf16* __r
     }
 }
 int posenc_tokens_nhwc(const void* x, int x_pitch, const float* pos, void* tokens, int B, int C, int H, int W, int pos_w, int oy, int ox,
-                       cudaStream_t st) {
+                       cudaStream_t st, const int* crop) {
     CFP_REQUIRE(C % 8 == 0 && x_pitch % 8 == 0 && C <= x_pitch, "posenc_tokens_nhwc: C = %d, pitch %d", C, x_pitch);
     const int64_t total = (int64_t)B * H * W * (C / 8);
     const int64_t want = (total + 255) / 256, cap = (int64_t)sm_count() * 16;
-    launch_pdl(posenc_tokens_nhwc_kernel, dim3((unsigned)(want < cap ? want : cap)), dim3(256), 0, st, (const bf16*)x, x_pitch, pos,
-               (bf16*)tokens, B, C, H, W, pos_w, oy, ox);
+    const dim3 grid((unsigned)(want < cap ? want : cap));
+    if (crop) {
+        launch_pdl(posenc_tokens_nhwc_kernel<true>, grid, dim3(256), 0, st, (const bf16*)x, x_pitch, pos, (bf16*)tokens, B, C, H, W,
+                   pos_w, 0, 0, crop);
+        return check_launch("posenc_tokens_nhwc_crop");
+    }
+    launch_pdl(posenc_tokens_nhwc_kernel<false>, grid, dim3(256), 0, st, (const bf16*)x, x_pitch, pos, (bf16*)tokens, B, C, H, W, pos_w,
+               oy, ox, (const int*)nullptr);
     return check_launch("posenc_tokens_nhwc");
 }
 

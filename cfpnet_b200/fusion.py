@@ -143,12 +143,16 @@ class TransformerFusion(nn.Module):
             raise ValueError(f"feat1 carries {S} samples per zone, positional_encodings2 has {self.positional_encodings2.shape[0]}")
         if tuple(kwargs["mask"].shape) != (B, g.zone_num ** 2):
             raise ValueError(f"mask {tuple(kwargs['mask'].shape)} is not [B={B}, zones={g.zone_num ** 2}]")
-        oy, ox = self.draw_crop(H, W)
+        # under a CUDA-graph capture the crop offsets live in device memory and the replay wrapper makes the draws
+        # (cfpnet_b200.pipeline.make_graphed_depth), as in forward()
+        crop_dev = self.__dict__.get("_crop_dev")
+        oy, ox = (0, 0) if crop_dev is not None else self.draw_crop(H, W)
         packed, pos, pos2, _buf = self._cache.get(self, self._pack)
         dev = x_tok.device
         code = _lib.dtype_code(dt)
-        posenc, copy = (("cfp_posenc_tokens_nhwc_f32_fwd", "cfp_copy_channels_f32") if dt == torch.float32
-                        else ("cfp_posenc_tokens_nhwc_fwd", "cfp_copy_channels"))
+        posenc, posenc_crop, copy = (
+            ("cfp_posenc_tokens_nhwc_f32_fwd", "cfp_posenc_tokens_nhwc_f32_crop_fwd", "cfp_copy_channels_f32") if dt == torch.float32
+            else ("cfp_posenc_tokens_nhwc_fwd", "cfp_posenc_tokens_nhwc_crop_fwd", "cfp_copy_channels"))
         feat1 = feat1.detach().to(dt).contiguous()
         mask = kwargs["mask"].to(device=dev, dtype=torch.uint8).contiguous()
         cg = _lib.CfpGeom.from_geometry(g)
@@ -160,8 +164,12 @@ class TransformerFusion(nn.Module):
                 dev.index, (dt, B, H, W), lambda t: t[0].numel() >= ws_bytes,
                 lambda: (torch.empty(ws_bytes, device=dev, dtype=torch.uint8), torch.empty(B, H * W, D, device=dev, dtype=dt)))
             st = _lib.stream_ptr()
-            _lib.call(posenc, x_tok.data_ptr(), x_pitch, pos, feat0.data_ptr(), B, D, H, W,
-                      self.max_resolution[0], self.max_resolution[1], oy, ox, st)
+            if crop_dev is not None:
+                _lib.call(posenc_crop, x_tok.data_ptr(), x_pitch, pos, feat0.data_ptr(), B, D, H, W,
+                          self.max_resolution[0], self.max_resolution[1], crop_dev.data_ptr(), st)
+            else:
+                _lib.call(posenc, x_tok.data_ptr(), x_pitch, pos, feat0.data_ptr(), B, D, H, W,
+                          self.max_resolution[0], self.max_resolution[1], oy, ox, st)
             self._run_layers(packed, pos2, feat0, feat1, mask, B, H, W, D, S, cg, work, ws_bytes, code, st, emb_copy)
             _lib.call(copy, feat0.data_ptr(), D, out_tok.data_ptr(), out_pitch, out_coff, D, B * H * W, st)
         return out_tok

@@ -106,6 +106,7 @@ class PackCache:
     def __init__(self, module: nn.Module = None):
         self._lock = threading.Lock()
         self._entries = {}                       # device -> (key, value)
+        self.generation = 0                      # bumped whenever a packed copy is dropped or replaced
 
     def __deepcopy__(self, memo):                # a copied / unpickled module starts with an empty cache
         return PackCache()
@@ -118,6 +119,12 @@ class PackCache:
         cfpnet_b200/train.py), which torch's version counters do not see."""
         with self._lock:
             self._entries.clear()
+            self.generation += 1
+
+    def held(self) -> list:
+        """The packed copies this cache holds now (a CUDA graph that reads them keeps them alive with this list)."""
+        with self._lock:
+            return list(self._entries.values())
 
     @staticmethod
     def _key(module: nn.Module):
@@ -136,6 +143,7 @@ class PackCache:
                 with torch.no_grad():
                     hit = (key, build())
                 self._entries[dev] = hit
+                self.generation += 1
             return hit[1]
 
 
@@ -153,6 +161,11 @@ class Scratch:
 
     def __reduce__(self):
         return (Scratch, ())
+
+    def held(self) -> list:
+        """The scratch tensors this module holds now (see PackCache.held)."""
+        with self._lock:
+            return list(self._entries.values())
 
     def get(self, device_index, key, fits, make):
         with self._lock:

@@ -8,14 +8,18 @@ adds the host<->device staging used for the end-to-end measurement.
 """
 from __future__ import annotations
 
+import itertools
+import operator
 from typing import Dict, Iterable, Iterator, List, Sequence, Tuple
 
 import torch
 import torch.nn as nn
 
+from . import _lib
 from .config import args
 from .encoder import HistogramEncoder
 from .fusion import TransformerFusion
+from .packing import PackCache, Scratch
 from .synth import LEVELS
 
 
@@ -260,3 +264,176 @@ class FusionPath(nn.Module):
             pending.append((i, si))
         while pending:
             yield drain(pending.pop(0))
+
+
+# ---------------------------------------------------------------------- the model below the image encoder as one CUDA graph
+# Counts every parameter, buffer and submodule registered anywhere (nn.Module.__setattr__, register_*, add_module,
+# load_state_dict(assign=True)): a capture guard walks its modules' whole tree only when this has moved since its last check.
+_REGISTRATIONS = [0]
+_hooks_installed = False
+
+
+def _count_registration(*_):
+    _REGISTRATIONS[0] += 1
+
+
+def _install_registration_hooks():
+    global _hooks_installed
+    if not _hooks_installed:
+        from torch.nn.modules import module as M
+        M.register_module_parameter_registration_hook(_count_registration)
+        M.register_module_buffer_registration_hook(_count_registration)
+        M.register_module_module_registration_hook(_count_registration)
+        _hooks_installed = True
+
+
+class _CaptureGuard:
+    """What a captured graph depends on beyond its own memory: the modules' parameters and buffers (the same tensors in the
+    same slots and, as PackCache keys them, the same ``data_ptr`` and ``_version``), their submodule tree, the packed-weight
+    copies the launches read (``PackCache.generation``), eval mode, the engine selection and the global flags the fusion calls
+    pass by value (``args.no_skip_inside``, ``args.change_embedding``).  ``check()`` raises ``CfpError`` when any of them has
+    changed since capture; ``held`` keeps the packed copies and scratch tensors the graph points at alive.
+
+    Per check, the tensors are compared through slots recorded at capture (C-level ``map`` over flat lists).  The tree itself
+    (which slots exist, which submodules hang where) is compared only when a registration happened somewhere since the last
+    check; ``nn.Module._apply`` (``.to()``, ``.half()``) writes the slot dicts without a registration and is caught by the
+    slot identity and ``data_ptr`` comparisons."""
+
+    def __init__(self, modules, decoder, hist_encoder):
+        _install_registration_hooks()
+        self.subs = [s for m in modules for s in m.modules()]
+        self.dicts = [d for s in self.subs for d in (s._parameters, s._buffers, s._modules)]
+        self.decoder, self.hist_encoder = decoder, hist_encoder
+        self.config = self._config()
+        self.registrations = _REGISTRATIONS[0]
+        self.slots = self._slots()
+        owned = [(d, n, t) for s in self.subs for d in (s._parameters, s._buffers) for n, t in d.items() if t is not None]
+        self.owners, self.names, self.tensors = [o[0] for o in owned], [o[1] for o in owned], [o[2] for o in owned]
+        self.ptrs, self.versions = self._ptrs(), self._versions()
+        stores = [v for s in self.subs for v in vars(s).values() if isinstance(v, (PackCache, Scratch))]
+        self.caches = [(c, c.generation) for c in stores if isinstance(c, PackCache) and c.held()]
+        self.held = [c.held() for c in stores]
+
+    def _config(self):
+        return self.decoder.compute_dtype, self.hist_encoder.out_dtype, bool(args.no_skip_inside), bool(args.change_embedding)
+
+    def _slots(self):
+        return list(itertools.chain.from_iterable(map(dict.values, self.dicts)))
+
+    def _ptrs(self):
+        return list(map(torch.Tensor.data_ptr, self.tensors))
+
+    def _versions(self):
+        return list(map(operator.attrgetter("_version"), self.tensors))
+
+    def check(self) -> None:
+        again = "; capture again with make_graphed_depth"
+        if any(map(operator.attrgetter("training"), self.subs)):
+            raise _lib.CfpError("a captured module is in training mode: the graph replays the eval-mode model" + again)
+        if self._config() != self.config:
+            raise _lib.CfpError("the engine or configuration changed since capture ((decoder.compute_dtype, hist_encoder.out_dtype, "
+                                f"args.no_skip_inside, args.change_embedding): {self.config} -> {self._config()})" + again)
+        replaced = not all(map(operator.is_, map(dict.get, self.owners, self.names), self.tensors))
+        if not replaced and _REGISTRATIONS[0] != self.registrations:
+            registrations = _REGISTRATIONS[0]
+            slots = self._slots()
+            replaced = len(slots) != len(self.slots) or not all(map(operator.is_, slots, self.slots))
+            if not replaced:
+                self.registrations = registrations
+        if replaced:
+            raise _lib.CfpError("a parameter, buffer or submodule of the captured modules was replaced since capture" + again)
+        if self._versions() != self.versions or self._ptrs() != self.ptrs:
+            raise _lib.CfpError("a parameter or buffer of the captured modules changed since capture (the graph reads the "
+                                "weights packed at capture)" + again)
+        if any(c.generation != g for c, g in self.caches):
+            raise _lib.CfpError("packed weights the graph reads were invalidated or re-packed since capture" + again)
+
+
+def make_graphed_depth(hist_encoder: HistogramEncoder, decoder, head, img_features: Sequence[torch.Tensor], hist_data: torch.Tensor,
+                       mask: torch.Tensor, patch_info, return_prob: bool = False, copy_inputs: bool = True):
+    """Capture the eval-mode model below the image encoder - ``hist_encoder(hist_data.unsqueeze(-1))`` ->
+    ``decoder.forward_nhwc`` -> ``head.forward_nhwc`` (deltar.py:40-61) - into one CUDA graph, in whichever engine the modules
+    are set up for (``decoder.compute_dtype``, ``hist_encoder.out_dtype``, the dtype of the ``cross_atten*`` modules), and
+    return ``run(img_features, hist_data, mask) -> (bin_edges, pred[, prob])`` that replays it: the 107-119 library launches of
+    an eager forward, each issued from Python through ctypes, become one graph launch.
+
+    ``img_features``: the five image-encoder maps [B, c, H/s, W/s] (s = 2 .. 32); ``hist_data`` [B, Z, S]; ``mask`` [B, Z];
+    all CUDA tensors.  ``copy_inputs``: ``run``'s arguments are copied into the captured static buffers first; with
+    ``copy_inputs=False`` the captured tensors ARE the inputs and ``run()`` takes no arguments (refill them in place).
+
+    The outputs are static tensors owned by the graph: every replay overwrites them (clone what must outlive the next call).
+    The graph is specific to the shapes (B, H, W), ``patch_info``, the engine and the global flags ``args.no_skip_inside`` /
+    ``args.change_embedding`` it was captured with.
+
+    Positional-encoding crops are not frozen: while capturing, the fusion modules read their offsets from a device buffer
+    (``cfp_posenc_tokens_nhwc_crop_fwd``), and every replay first makes the reference's draws from torch's global generator
+    in the decoder's order (``cross_atten3``, ``2``, ``1``; oy then ox; nothing drawn along an axis the map fills) and
+    uploads them with a stream-ordered copy, so the generator advances exactly as in an eager forward.
+
+    Ownership and staleness: ``run`` keeps the fusion modules' scratch tensors and every packed-weight copy the graph reads
+    alive, so an eager call at another shape or a re-pack cannot free memory under it.  ``run`` raises ``CfpError`` instead
+    of replaying when a parameter or buffer of the three modules changed since capture (``data_ptr`` / ``_version``, or a
+    replaced tensor or submodule), when a ``PackCache`` of theirs was invalidated (``FlatTrainer.update``) or re-packed,
+    when a module is in ``.train()`` mode, or when ``decoder.compute_dtype`` / ``hist_encoder.out_dtype`` /
+    ``args.no_skip_inside`` / ``args.change_embedding`` changed: capture again.  ``run.check()`` is that test alone."""
+    mods = (hist_encoder, decoder, head)
+    if any(s.training for m in mods for s in m.modules()):
+        raise _lib.CfpError("make_graphed_depth captures the eval-mode model: call .eval() on the histogram encoder, decoder and head")
+    if len(img_features) != 5:
+        raise ValueError(f"img_features holds the five image-encoder maps, got {len(img_features)}")
+    inputs = [*img_features, hist_data, mask]
+    for t in inputs:
+        _lib.require_cuda(t, "make_graphed_depth inputs")
+    static = [t.clone() for t in inputs] if copy_inputs else list(inputs)
+    dev = hist_data.device
+    fusions = (decoder.cross_atten3, decoder.cross_atten2, decoder.cross_atten1)
+    # each fusion call runs at the size of the skip feature its level is upsampled to (decoder.py:109-121)
+    shapes = [(m, int(x.shape[2]), int(x.shape[3])) for m, x in zip(fusions, (static[3], static[2], static[1]))]
+    for m, H, W in shapes:
+        if H > m.max_resolution[0] or W > m.max_resolution[1]:
+            raise ValueError("feature map larger than the positional-encoding table")
+    draws = any(H < m.max_resolution[0] or W < m.max_resolution[1] for m, H, W in shapes)
+    crop_dev = torch.zeros(3, 2, device=dev, dtype=torch.int32)
+
+    def forward():
+        hist = hist_encoder(static[5].unsqueeze(-1))
+        unet, H, W = decoder.forward_nhwc(static[:5], hist, rect_data=None, mask=static[6], patch_info=patch_info, rgb=None)
+        return head.forward_nhwc(unet, H, W, return_prob=return_prob)
+
+    side = torch.cuda.Stream(dev)
+    side.wait_stream(torch.cuda.current_stream(dev))
+    try:
+        for i, m in enumerate(fusions):
+            m.__dict__["_crop_dev"] = crop_dev[i]
+        with torch.cuda.device(dev), torch.cuda.stream(side), torch.no_grad():   # warm-up off the capture: packing, scratch,
+            for _ in range(2):                                                      # smem attributes
+                forward()
+        torch.cuda.current_stream(dev).wait_stream(side)
+        guard = _CaptureGuard(mods, decoder, hist_encoder)
+        graph = torch.cuda.CUDAGraph()
+        with torch.cuda.device(dev), torch.cuda.graph(graph), torch.no_grad():
+            outs = forward()
+        guard.check()                            # nothing was re-packed or re-allocated while capturing
+    finally:
+        for m in fusions:
+            m.__dict__.pop("_crop_dev", None)
+
+    def run(*args):
+        guard.check()
+        if copy_inputs:
+            feats, hd, mk = args
+            src = [*feats, hd, mk]
+            if len(src) != len(static) or any(a.shape != b.shape for a, b in zip(src, static)):
+                raise ValueError("run() takes inputs shaped like the captured ones: the graph is specific to its shapes")
+            for dst, x in zip(static, src):
+                dst.copy_(x, non_blocking=True)
+        elif args:
+            raise TypeError("captured with copy_inputs=False: run() takes no arguments (refill the captured tensors in place)")
+        if draws:
+            vals = torch.tensor([m.draw_crop(H, W) for m, H, W in shapes], dtype=torch.int32)
+            crop_dev.copy_(vals, non_blocking=True)   # stream-ordered before the replay; the host copy is staged at the call
+        graph.replay()
+        return outs
+
+    run.graph, run.crop_dev, run.static, run.check, run.guard = graph, crop_dev, static, guard.check, guard
+    return run

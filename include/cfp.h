@@ -312,6 +312,11 @@ CFP_API int cfp_upsample_concat(const void *lo, int h, int w, int c_lo, int lo_p
 /* cfp_posenc_tokens_fwd for a caller that already holds the map channels-last (bf16, pitch x_pitch): tokens = x + pos crop. */
 CFP_API int cfp_posenc_tokens_nhwc_fwd(const void *x, int x_pitch, const float *pos, void *tokens, int B, int C, int H, int W,
                                        int pos_h, int pos_w, int oy, int ox, void *stream);
+/* cfp_posenc_tokens_nhwc_fwd with the crop offsets (oy, ox) read from DEVICE memory (crop [2], int32) when the kernel runs, as
+ * cfp_posenc_tokens_crop_fwd: a CUDA-graph replay of the decoder takes fresh offsets from the buffer.  The host cannot see the
+ * offsets and does not range-check them: the caller keeps 0 <= oy <= pos_h - H, 0 <= ox <= pos_w - W. */
+CFP_API int cfp_posenc_tokens_nhwc_crop_fwd(const void *x, int x_pitch, const float *pos, void *tokens, int B, int C, int H, int W,
+                                            int pos_h, int pos_w, const int *crop, void *stream);
 CFP_API int cfp_copy_channels(const void *src, int src_pitch, void *dst, int dst_pitch, int coff, int C, int64_t rows, void *stream);
 CFP_API int cfp_head_bins(const void *x, int pitch, int B, int npix, int E, const float *wc, const float *w0, const float *b0,
                           const float *w2, const float *b2, const float *w4, const float *b4, int hidden, int n_bins, float min_val,
@@ -336,6 +341,9 @@ CFP_API int cfp_upsample_concat_f32(const float *lo, int h, int w, int c_lo, int
                                     int B, int H, int W, int c_out, void *stream);
 CFP_API int cfp_posenc_tokens_nhwc_f32_fwd(const float *x, int x_pitch, const float *pos, float *tokens, int B, int C, int H, int W,
                                            int pos_h, int pos_w, int oy, int ox, void *stream);
+/* The fp32 form of cfp_posenc_tokens_nhwc_crop_fwd (same contract: the caller keeps the crop inside the table). */
+CFP_API int cfp_posenc_tokens_nhwc_f32_crop_fwd(const float *x, int x_pitch, const float *pos, float *tokens, int B, int C, int H,
+                                                int W, int pos_h, int pos_w, const int *crop, void *stream);
 CFP_API int cfp_copy_channels_f32(const float *src, int src_pitch, float *dst, int dst_pitch, int coff, int C, int64_t rows,
                                   void *stream);
 CFP_API int cfp_head_bins_f32(const float *x, int pitch, int B, int npix, int E, const float *wc, const float *w0, const float *b0,
