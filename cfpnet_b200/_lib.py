@@ -18,7 +18,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CFP_LIB_PATH") or os.path.join(_HERE, "libcfp.so")   # override: debug builds (tools/)
 
 CFP_F32, CFP_BF16 = 0, 1
-ABI_VERSION = 15
+ABI_VERSION = 16
 _fp = C.POINTER(C.c_float)
 
 
@@ -65,7 +65,7 @@ SIGNATURES = {
     "cfp_geometry_from_rects": (_i, [_fp, _i, _i, _i, _i, _i, C.POINTER(CfpGeom)]),
     "cfp_hist_encoder_fwd": (_i, [_p, _p, _p, _p, _i64, C.POINTER(CfpHistW), _i, _p]),
     "cfp_zone_masks": (_i, [_p, _p, _p, _p, _i, _i, _i, C.POINTER(CfpGeom), _p]),
-    "cfp_posenc_tokens_fwd": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p]),
+    "cfp_posenc_tokens_fwd": (_i, [_p, _p, _p] + [_i] * 8 + [_p, _i, _p]),
     "cfp_tokens_to_nchw": (_i, [_p, _p, _i, _i, _i, _i, _i, _p]),
     "cfp_d2i_fwd": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, C.POINTER(CfpGeom),
                          C.POINTER(CfpLoftrW), _i, _p, _sz, _i, _p]),
@@ -91,21 +91,12 @@ SIGNATURES = {
     "cfp_tr_dwconv_wgrad": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _p]),
     "cfp_tr_sumsq": (_i, [_p, _i64, C.c_float, _p, _p]),
     "cfp_tr_adamw": (_i, [_p, _p, _p, _p, _i64, _p, _p, _i] + [C.c_float] * 4 + [_i, C.c_float, _p, C.c_float, _p]),
-    "cfp_conv_fwd": (_i, [_p] + [_i] * 7 + [_p, _p, C.c_float, _p, _i, _i, _p]),
-    "cfp_upsample_concat": (_i, [_p, _i, _i, _i, _i, _p, _i, _p, _i, _i, _i, _i, _p]),
-    "cfp_posenc_tokens_crop_fwd": (_i, [_p, _p, _p] + [_i] * 6 + [_p, _i, _p]),
-    "cfp_posenc_tokens_nhwc_fwd": (_i, [_p, _i, _p, _p] + [_i] * 8 + [_p]),
-    "cfp_posenc_tokens_nhwc_crop_fwd": (_i, [_p, _i, _p, _p] + [_i] * 6 + [_p, _p]),
-    "cfp_copy_channels": (_i, [_p, _i, _p, _i, _i, _i, _i64, _p]),
-    "cfp_head_bins": (_i, [_p, _i, _i, _i, _i] + [_p] * 7 + [_i, _i, C.c_float, C.c_float, _p, _p, _p, _p]),
-    "cfp_head_expect": (_i, [_p, _i, _i, _i, _p, _p, _p, _i, _p, _p, _p]),
-    "cfp_conv_f32_fwd": (_i, [_p] + [_i] * 6 + [_p, _p, C.c_float, _p, _i, _i, _p]),
-    "cfp_upsample_concat_f32": (_i, [_p, _i, _i, _i, _i, _p, _i, _p, _i, _i, _i, _i, _p]),
-    "cfp_posenc_tokens_nhwc_f32_fwd": (_i, [_p, _i, _p, _p] + [_i] * 8 + [_p]),
-    "cfp_posenc_tokens_nhwc_f32_crop_fwd": (_i, [_p, _i, _p, _p] + [_i] * 6 + [_p, _p]),
-    "cfp_copy_channels_f32": (_i, [_p, _i, _p, _i, _i, _i, _i64, _p]),
-    "cfp_head_bins_f32": (_i, [_p, _i, _i, _i, _i] + [_p] * 7 + [_i, _i, C.c_float, C.c_float, _p, _p, _p, _p]),
-    "cfp_head_expect_f32": (_i, [_p, _i, _i, _i, _p, _p, _p, _i, _p, _p, _p]),
+    "cfp_conv_fwd": (_i, [_p] + [_i] * 7 + [_p, _p, C.c_float, _p, _i, _i, _i, _p]),
+    "cfp_upsample_concat": (_i, [_p, _i, _i, _i, _i, _p, _i, _p, _i, _i, _i, _i, _i, _p]),
+    "cfp_posenc_tokens_nhwc_fwd": (_i, [_p, _i, _p, _p] + [_i] * 8 + [_p, _i, _p]),
+    "cfp_copy_channels": (_i, [_p, _i, _p, _i, _i, _i, _i64, _i, _p]),
+    "cfp_head_bins": (_i, [_p, _i, _i, _i, _i] + [_p] * 7 + [_i, _i, C.c_float, C.c_float, _p, _p, _p, _i, _p]),
+    "cfp_head_expect": (_i, [_p, _i, _i, _i, _p, _p, _p, _i, _p, _p, _i, _p]),
     "cfp_tr_conv_wgrad_scratch_floats": (_sz, [_i] * 6),
     "cfp_tr_conv_wgrad_f32": (_i, [_p, _p, _p, _p] + [_i] * 6 + [_p]),
     "cfp_tr_upsample_concat_bwd_f32": (_i, [_p, _i, _p, _i, _i, _i, _p, _i, _i, _i, _i, _p]),

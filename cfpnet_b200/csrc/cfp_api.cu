@@ -243,25 +243,28 @@ CFP_API int cfp_zone_masks(const uint8_t* mask, uint8_t* zone_mask, uint8_t* his
     return zone_masks(mask, zone_mask, hist_mask, pad_mask, B, H, W, *g, (cudaStream_t)stream);
 }
 
+// The positional-encoding crop of an H x W map in the pos_h x pos_w table.  Host offsets (crop == NULL) must lie inside
+// it.  Device offsets are read when the kernel runs, so only the map's size can be checked, and host offsets passed
+// beside them would be ignored: they must be 0.
+static int check_crop(int H, int W, int pos_h, int pos_w, int oy, int ox, const int* crop) {
+    if (crop == nullptr) {
+        CFP_REQUIRE(oy >= 0 && ox >= 0 && ox + W <= pos_w && oy + H <= pos_h,
+                    "positional-encoding crop [%d:%d,%d:%d] outside the %dx%d table", oy, oy + H, ox, ox + W, pos_h, pos_w);
+        return 0;
+    }
+    CFP_REQUIRE(W <= pos_w && H <= pos_h, "feature map %dx%d larger than the %dx%d positional-encoding table", H, W, pos_h, pos_w);
+    CFP_REQUIRE(oy == 0 && ox == 0, "host crop offsets (%d, %d) given with a device crop buffer: pass 0, 0", oy, ox);
+    return 0;
+}
+
 CFP_API int cfp_posenc_tokens_fwd(const void* x_nchw, const float* pos, void* tokens, int B, int C, int H, int W, int pos_h,
-                          int pos_w, int oy, int ox, int dtype, void* stream) {
+                          int pos_w, int oy, int ox, const int* crop, int dtype, void* stream) {
     begin_call(stream);
     CFP_REQUIRE(x_nchw && pos && tokens, "null pointer");
     CFP_REQUIRE(B > 0 && B <= 65535 && C > 0 && H > 0 && W > 0, "bad shape");
-    CFP_REQUIRE(oy >= 0 && ox >= 0 && ox + W <= pos_w && oy + H <= pos_h,
-                "positional-encoding crop [%d:%d,%d:%d] outside the %dx%d table", oy, oy + H, ox, ox + W, pos_h, pos_w);
+    if (int e = check_crop(H, W, pos_h, pos_w, oy, ox, crop)) return e;
     CFP_REQUIRE(dtype == CFP_F32 || dtype == CFP_BF16, "unsupported dtype %d", dtype);
-    return posenc_tokens(x_nchw, pos, tokens, B, C, H, W, pos_w, oy, ox, dtype, (cudaStream_t)stream);
-}
-
-CFP_API int cfp_posenc_tokens_crop_fwd(const void* x_nchw, const float* pos, void* tokens, int B, int C, int H, int W, int pos_h,
-                                       int pos_w, const int* crop, int dtype, void* stream) {
-    begin_call(stream);
-    CFP_REQUIRE(x_nchw && pos && tokens && crop, "null pointer");
-    CFP_REQUIRE(B > 0 && B <= 65535 && C > 0 && H > 0 && W > 0, "bad shape");
-    CFP_REQUIRE(W <= pos_w && H <= pos_h, "feature map %dx%d larger than the %dx%d positional-encoding table", H, W, pos_h, pos_w);
-    CFP_REQUIRE(dtype == CFP_F32 || dtype == CFP_BF16, "unsupported dtype %d", dtype);
-    return posenc_tokens(x_nchw, pos, tokens, B, C, H, W, pos_w, 0, 0, dtype, (cudaStream_t)stream, crop);
+    return posenc_tokens(x_nchw, pos, tokens, B, C, H, W, pos_w, oy, ox, dtype, (cudaStream_t)stream, crop);
 }
 
 CFP_API int cfp_tokens_to_nchw(const void* tokens, void* out_nchw, int B, int C, int H, int W, int dtype, void* stream) {
@@ -507,107 +510,68 @@ CFP_API int cfp_depth_metrics(const float* gt, const float* pred, const uint8_t*
 }
 
 // ---------------------------------------------------------------- decoder shell (f1) and adaptive-bins head (f2)
-CFP_API int cfp_conv_fwd(const void* in, int B, int H, int W, int cin, int cout, int ksize, int kchunk, const void* w_tc,
-                         const float* shift, float leaky_slope, void* out, int out_pitch, int out_coff, void* stream) {
-    begin_call(stream);
-    CFP_REQUIRE(in && w_tc && shift && out, "null pointer");
-    CFP_REQUIRE(ksize == 1 || ksize == 3, "kernel size %d (1 and 3 are served)", ksize);
-    return conv_gen_tc(in, cin, kchunk, ksize * ksize, w_tc, shift, leaky_slope, out, out_pitch, out_coff, B, H, W, cout, (cudaStream_t)stream);
-}
-CFP_API int cfp_upsample_concat(const void* lo, int h, int w, int c_lo, int lo_pitch, const float* skip, int c_skip, void* out, int B,
-                                int H, int W, int c_out, void* stream) {
-    begin_call(stream);
-    CFP_REQUIRE(out, "null pointer");
-    return upsample_concat(lo, h, w, c_lo, lo_pitch, skip, c_skip, out, B, H, W, c_out, (cudaStream_t)stream);
-}
-CFP_API int cfp_posenc_tokens_nhwc_fwd(const void* x, int x_pitch, const float* pos, void* tokens, int B, int C, int H, int W,
-                                       int pos_h, int pos_w, int oy, int ox, void* stream) {
-    begin_call(stream);
-    CFP_REQUIRE(x && pos && tokens, "null pointer");
-    CFP_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, "bad shape");
-    CFP_REQUIRE(oy >= 0 && ox >= 0 && ox + W <= pos_w && oy + H <= pos_h,
-                "positional-encoding crop [%d:%d,%d:%d] outside the %dx%d table", oy, oy + H, ox, ox + W, pos_h, pos_w);
-    return posenc_tokens_nhwc(x, x_pitch, pos, tokens, B, C, H, W, pos_w, oy, ox, (cudaStream_t)stream);
-}
-CFP_API int cfp_posenc_tokens_nhwc_crop_fwd(const void* x, int x_pitch, const float* pos, void* tokens, int B, int C, int H, int W,
-                                            int pos_h, int pos_w, const int* crop, void* stream) {
-    begin_call(stream);
-    CFP_REQUIRE(x && pos && tokens && crop, "null pointer");
-    CFP_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, "bad shape");
-    CFP_REQUIRE(W <= pos_w && H <= pos_h, "feature map %dx%d larger than the %dx%d positional-encoding table", H, W, pos_h, pos_w);
-    return posenc_tokens_nhwc(x, x_pitch, pos, tokens, B, C, H, W, pos_w, 0, 0, (cudaStream_t)stream, crop);
-}
-CFP_API int cfp_copy_channels(const void* src, int src_pitch, void* dst, int dst_pitch, int coff, int C, int64_t rows, void* stream) {
-    begin_call(stream);
-    CFP_REQUIRE(src && dst && rows >= 0, "bad arguments");
-    return copy_channels(src, src_pitch, dst, dst_pitch, coff, C, rows, (cudaStream_t)stream);
-}
-CFP_API int cfp_head_bins(const void* x, int pitch, int B, int npix, int E, const float* wc, const float* w0, const float* b0,
-                          const float* w2, const float* b2, const float* w4, const float* b4, int hidden, int n_bins, float min_val,
-                          float max_val, float* mean_scratch, float* edges, float* centres, void* stream) {
-    begin_call(stream);
-    CFP_REQUIRE(x && wc && w0 && b0 && w2 && b2 && w4 && b4 && mean_scratch && edges && centres, "null pointer");
-    if (int e = channel_mean(x, pitch, E, B, npix, mean_scratch, (cudaStream_t)stream)) return e;
-    return head_regressor(mean_scratch, wc, w0, b0, w2, b2, w4, b4, B, E, hidden, n_bins, min_val, max_val, edges, centres,
-                          (cudaStream_t)stream);
-}
-CFP_API int cfp_head_expect(const void* x, int pitch, int B, int npix, const void* w_tc, const float* bias, const float* centres,
-                            int n_bins, float* pred, float* prob, void* stream) {
-    begin_call(stream);
-    CFP_REQUIRE(x && w_tc && bias && centres && pred, "null pointer");
-    return head_expect_tc(x, pitch, B, npix, w_tc, bias, centres, n_bins, pred, prob, (cudaStream_t)stream);
-}
-
-// the exact fp32 engine of the same stages (k_dec_f32.cu)
-CFP_API int cfp_conv_f32_fwd(const float* in, int B, int H, int W, int cin, int cout, int ksize, const float* w, const float* shift,
-                             float leaky_slope, float* out, int out_pitch, int out_coff, void* stream) {
+// CFP_BF16 runs the tcgen05 engine (k_dec_tc.cu), CFP_F32 the exact fp32 engine (k_dec_f32.cu).
+CFP_API int cfp_conv_fwd(const void* in, int B, int H, int W, int cin, int cout, int ksize, int kchunk, const void* w,
+                         const float* shift, float leaky_slope, void* out, int out_pitch, int out_coff, int dtype, void* stream) {
     begin_call(stream);
     CFP_REQUIRE(in && w && shift && out, "null pointer");
     CFP_REQUIRE(ksize == 1 || ksize == 3, "kernel size %d (1 and 3 are served)", ksize);
-    return conv_f32(in, cin, ksize * ksize, w, shift, leaky_slope, out, out_pitch, out_coff, B, H, W, cout, (cudaStream_t)stream);
+    CFP_REQUIRE(dtype == CFP_F32 || dtype == CFP_BF16, "unsupported dtype %d", dtype);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == CFP_BF16)
+        return conv_gen_tc(in, cin, kchunk, ksize * ksize, w, shift, leaky_slope, out, out_pitch, out_coff, B, H, W, cout, st);
+    CFP_REQUIRE(kchunk == 0, "kchunk %d: the fp32 convolution stages no K-chunks (pass 0)", kchunk);
+    return conv_f32((const float*)in, cin, ksize * ksize, (const float*)w, shift, leaky_slope, (float*)out, out_pitch, out_coff, B, H, W,
+                    cout, st);
 }
-CFP_API int cfp_upsample_concat_f32(const float* lo, int h, int w, int c_lo, int lo_pitch, const float* skip, int c_skip, float* out, int B,
-                                    int H, int W, int c_out, void* stream) {
+CFP_API int cfp_upsample_concat(const void* lo, int h, int w, int c_lo, int lo_pitch, const float* skip, int c_skip, void* out, int B,
+                                int H, int W, int c_out, int dtype, void* stream) {
     begin_call(stream);
     CFP_REQUIRE(out, "null pointer");
-    return upsample_concat_f32(lo, h, w, c_lo, lo_pitch, skip, c_skip, out, B, H, W, c_out, (cudaStream_t)stream);
+    CFP_REQUIRE(dtype == CFP_F32 || dtype == CFP_BF16, "unsupported dtype %d", dtype);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == CFP_BF16) return upsample_concat(lo, h, w, c_lo, lo_pitch, skip, c_skip, out, B, H, W, c_out, st);
+    return upsample_concat_f32((const float*)lo, h, w, c_lo, lo_pitch, skip, c_skip, (float*)out, B, H, W, c_out, st);
 }
-CFP_API int cfp_posenc_tokens_nhwc_f32_fwd(const float* x, int x_pitch, const float* pos, float* tokens, int B, int C, int H, int W,
-                                           int pos_h, int pos_w, int oy, int ox, void* stream) {
+CFP_API int cfp_posenc_tokens_nhwc_fwd(const void* x, int x_pitch, const float* pos, void* tokens, int B, int C, int H, int W,
+                                       int pos_h, int pos_w, int oy, int ox, const int* crop, int dtype, void* stream) {
     begin_call(stream);
     CFP_REQUIRE(x && pos && tokens, "null pointer");
     CFP_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, "bad shape");
-    CFP_REQUIRE(oy >= 0 && ox >= 0 && ox + W <= pos_w && oy + H <= pos_h,
-                "positional-encoding crop [%d:%d,%d:%d] outside the %dx%d table", oy, oy + H, ox, ox + W, pos_h, pos_w);
-    return posenc_tokens_nhwc_f32(x, x_pitch, pos, tokens, B, C, H, W, pos_w, oy, ox, (cudaStream_t)stream);
+    if (int e = check_crop(H, W, pos_h, pos_w, oy, ox, crop)) return e;
+    CFP_REQUIRE(dtype == CFP_F32 || dtype == CFP_BF16, "unsupported dtype %d", dtype);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == CFP_BF16) return posenc_tokens_nhwc(x, x_pitch, pos, tokens, B, C, H, W, pos_w, oy, ox, st, crop);
+    return posenc_tokens_nhwc_f32((const float*)x, x_pitch, pos, (float*)tokens, B, C, H, W, pos_w, oy, ox, st, crop);
 }
-CFP_API int cfp_posenc_tokens_nhwc_f32_crop_fwd(const float* x, int x_pitch, const float* pos, float* tokens, int B, int C, int H,
-                                                int W, int pos_h, int pos_w, const int* crop, void* stream) {
-    begin_call(stream);
-    CFP_REQUIRE(x && pos && tokens && crop, "null pointer");
-    CFP_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, "bad shape");
-    CFP_REQUIRE(W <= pos_w && H <= pos_h, "feature map %dx%d larger than the %dx%d positional-encoding table", H, W, pos_h, pos_w);
-    return posenc_tokens_nhwc_f32(x, x_pitch, pos, tokens, B, C, H, W, pos_w, 0, 0, (cudaStream_t)stream, crop);
-}
-CFP_API int cfp_copy_channels_f32(const float* src, int src_pitch, float* dst, int dst_pitch, int coff, int C, int64_t rows, void* stream) {
+CFP_API int cfp_copy_channels(const void* src, int src_pitch, void* dst, int dst_pitch, int coff, int C, int64_t rows, int dtype,
+                              void* stream) {
     begin_call(stream);
     CFP_REQUIRE(src && dst && rows >= 0, "bad arguments");
-    return copy_channels_f32(src, src_pitch, dst, dst_pitch, coff, C, rows, (cudaStream_t)stream);
+    CFP_REQUIRE(dtype == CFP_F32 || dtype == CFP_BF16, "unsupported dtype %d", dtype);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == CFP_BF16) return copy_channels(src, src_pitch, dst, dst_pitch, coff, C, rows, st);
+    return copy_channels_f32((const float*)src, src_pitch, (float*)dst, dst_pitch, coff, C, rows, st);
 }
-CFP_API int cfp_head_bins_f32(const float* x, int pitch, int B, int npix, int E, const float* wc, const float* w0, const float* b0,
-                              const float* w2, const float* b2, const float* w4, const float* b4, int hidden, int n_bins, float min_val,
-                              float max_val, float* mean_scratch, float* edges, float* centres, void* stream) {
+CFP_API int cfp_head_bins(const void* x, int pitch, int B, int npix, int E, const float* wc, const float* w0, const float* b0,
+                          const float* w2, const float* b2, const float* w4, const float* b4, int hidden, int n_bins, float min_val,
+                          float max_val, float* mean_scratch, float* edges, float* centres, int dtype, void* stream) {
     begin_call(stream);
     CFP_REQUIRE(x && wc && w0 && b0 && w2 && b2 && w4 && b4 && mean_scratch && edges && centres, "null pointer");
-    if (int e = channel_mean_f32(x, pitch, E, B, npix, mean_scratch, (cudaStream_t)stream)) return e;
-    return head_regressor(mean_scratch, wc, w0, b0, w2, b2, w4, b4, B, E, hidden, n_bins, min_val, max_val, edges, centres,
-                          (cudaStream_t)stream);
+    CFP_REQUIRE(dtype == CFP_F32 || dtype == CFP_BF16, "unsupported dtype %d", dtype);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (int e = dtype == CFP_BF16 ? channel_mean(x, pitch, E, B, npix, mean_scratch, st)
+                                  : channel_mean_f32((const float*)x, pitch, E, B, npix, mean_scratch, st)) return e;
+    return head_regressor(mean_scratch, wc, w0, b0, w2, b2, w4, b4, B, E, hidden, n_bins, min_val, max_val, edges, centres, st);
 }
-CFP_API int cfp_head_expect_f32(const float* x, int pitch, int B, int npix, const float* w_t, const float* bias, const float* centres,
-                                int n_bins, float* pred, float* prob, void* stream) {
+CFP_API int cfp_head_expect(const void* x, int pitch, int B, int npix, const void* w, const float* bias, const float* centres,
+                            int n_bins, float* pred, float* prob, int dtype, void* stream) {
     begin_call(stream);
-    CFP_REQUIRE(x && w_t && bias && centres && pred, "null pointer");
-    return head_expect_f32(x, pitch, B, npix, w_t, bias, centres, n_bins, pred, prob, (cudaStream_t)stream);
+    CFP_REQUIRE(x && w && bias && centres && pred, "null pointer");
+    CFP_REQUIRE(dtype == CFP_F32 || dtype == CFP_BF16, "unsupported dtype %d", dtype);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == CFP_BF16) return head_expect_tc(x, pitch, B, npix, w, bias, centres, n_bins, pred, prob, st);
+    return head_expect_f32((const float*)x, pitch, B, npix, (const float*)w, bias, centres, n_bins, pred, prob, st);
 }
 
 // the decoder shell and head in train mode (k_dec_train.cu)

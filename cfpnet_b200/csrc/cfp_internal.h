@@ -23,7 +23,7 @@ inline size_t elem_size(int dtype) { return dtype == CFP_F32 ? 4 : 2; }
 
 // k_layout.cu
 int posenc_tokens(const void* x, const float* pos, void* tokens, int B, int C, int H, int W, int pos_w,
-                  int oy, int ox, int dtype, cudaStream_t st, const int* crop = nullptr);
+                  int oy, int ox, int dtype, cudaStream_t st, const int* crop);
 int tokens_to_nchw(const void* tokens, void* out, int B, int C, int H, int W, int dtype, cudaStream_t st);
 int zone_masks(const uint8_t* mask, uint8_t* zm, uint8_t* hm, uint8_t* pm, int B, int H, int W,
                const cfp_geom& g, cudaStream_t st);
@@ -122,7 +122,7 @@ int upsample_concat(const void* lo, int h, int w, int c_lo, int lo_pitch, const 
 int copy_channels(const void* src, int src_pitch, void* dst, int dst_pitch, int coff, int C, int64_t rows, cudaStream_t st);
 // crop (device int32 [2]) non-null: the offsets are read from it when the kernel runs and oy / ox are ignored
 int posenc_tokens_nhwc(const void* x, int x_pitch, const float* pos, void* tokens, int B, int C, int H, int W, int pos_w, int oy, int ox,
-                       cudaStream_t st, const int* crop = nullptr);
+                       cudaStream_t st, const int* crop);
 int channel_mean(const void* x, int pitch, int C, int B, int npix, float* mean, cudaStream_t st);
 int head_regressor(const float* mean, const float* wc, const float* w0, const float* b0, const float* w2, const float* b2, const float* w4,
                    const float* b4, int B, int E, int Hd, int nb, float min_val, float max_val, float* edges, float* centres,
@@ -137,7 +137,7 @@ int upsample_concat_f32(const float* lo, int h, int w, int c_lo, int lo_pitch, c
                         int c_out, cudaStream_t st);
 int copy_channels_f32(const float* src, int src_pitch, float* dst, int dst_pitch, int coff, int C, int64_t rows, cudaStream_t st);
 int posenc_tokens_nhwc_f32(const float* x, int x_pitch, const float* pos, float* tokens, int B, int C, int H, int W, int pos_w, int oy, int ox,
-                           cudaStream_t st, const int* crop = nullptr);
+                           cudaStream_t st, const int* crop);
 int channel_mean_f32(const float* x, int pitch, int C, int B, int npix, float* mean, cudaStream_t st);
 int head_expect_f32(const float* x, int pitch, int B, int npix, const float* w_t, const float* bias, const float* centres, int nb, float* pred,
                     float* prob, cudaStream_t st);

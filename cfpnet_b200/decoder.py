@@ -7,9 +7,9 @@ checkpoint loads with ``strict=True``.  The maps stay channels-last bf16 between
 the fusion layers): every ``torch.cat`` of the reference is a write into a slice of a wider buffer, the bilinear
 upsample + skip concat is one kernel, convs are ``cfp_conv_fwd`` (tcgen05 implicit GEMM with the eval-mode BatchNorm folded
 and LeakyReLU in the epilogue), and ``conv_out`` + softmax + bin expectation is ``cfp_head_expect`` (the 256-bin
-probability volume is only written on request).  The fp32 engine runs the same sequence on fp32 maps through
-the ``*_f32`` kernels (FFMA, fixed summation order) and the fusion modules' fp32 engine.  In ``.train()`` mode ``forward``
-runs the fp32 training path of cfpnet_b200/decoder_train.py.  No CPU fallback.
+probability volume is only written on request).  The fp32 engine runs the same sequence on fp32 maps through the
+same entry points with ``CFP_F32`` (FFMA, fixed summation order) and the fusion modules' fp32 engine.  In ``.train()``
+mode ``forward`` runs the fp32 training path of cfpnet_b200/decoder_train.py.  No CPU fallback.
 """
 from __future__ import annotations
 
@@ -52,8 +52,8 @@ def _conv_plan(cin: int, cout: int, may_pad: bool) -> Tuple[int, int]:
 
 
 class _PackedConv:
-    """One conv (+ folded BatchNorm) packed for cfp_conv_fwd: bf16 blocks [chunk][tap][kc/8][cout][8] + fp32 shift; with
-    ``dtype=torch.float32`` for cfp_conv_f32_fwd: fp32 [tap][cin][cout], input channels not padded."""
+    """One conv (+ folded BatchNorm) packed for cfp_conv_fwd: ``w`` = bf16 blocks [chunk][tap][kc/8][cout][8], + fp32 shift;
+    with ``dtype=torch.float32``: ``w`` = fp32 [tap][cin][cout], input channels not padded, kc = 0 (no K-chunks)."""
 
     def __init__(self, conv: nn.Conv2d, bn: nn.BatchNorm2d | None, device, may_pad: bool = False, dtype=torch.bfloat16):
         w = host(conv.weight)                                              # [cout, cin, k, k]
@@ -76,7 +76,7 @@ class _PackedConv:
         wp[:, :cin] = w
         blocks = [umma_block(wp[:, c0:c0 + self.kc, ky, kx]) for c0 in range(0, self.cin_pad, self.kc)
                   for ky in range(k) for kx in range(k)]
-        self.w_tc = torch.stack(blocks).contiguous().to(device)
+        self.w = torch.stack(blocks).contiguous().to(device)
 
 
 class UpSampleBN(nn.Module):
@@ -91,12 +91,8 @@ class UpSampleBN(nn.Module):
 
 
 def _conv(pc: _PackedConv, x: torch.Tensor, B: int, H: int, W: int, slope: float, out: torch.Tensor, out_pitch: int, out_coff: int):
-    if pc.dtype == torch.float32:
-        _lib.call("cfp_conv_f32_fwd", x.data_ptr(), B, H, W, pc.cin, pc.cout, pc.k, pc.w.data_ptr(), pc.shift.data_ptr(),
-                  C.c_float(slope), out.data_ptr(), out_pitch, out_coff, _lib.stream_ptr())
-        return
-    _lib.call("cfp_conv_fwd", x.data_ptr(), B, H, W, pc.cin_pad, pc.cout, pc.k, pc.kc, pc.w_tc.data_ptr(), pc.shift.data_ptr(),
-              C.c_float(slope), out.data_ptr(), out_pitch, out_coff, _lib.stream_ptr())
+    _lib.call("cfp_conv_fwd", x.data_ptr(), B, H, W, pc.cin_pad, pc.cout, pc.k, pc.kc, pc.w.data_ptr(), pc.shift.data_ptr(),
+              C.c_float(slope), out.data_ptr(), out_pitch, out_coff, _lib.dtype_code(pc.dtype), _lib.stream_ptr())
 
 
 class Decoder(nn.Module):
@@ -162,8 +158,7 @@ class Decoder(nn.Module):
         dt = self.compute_dtype
         if dt not in (torch.bfloat16, torch.float32):
             raise ValueError(f"Decoder.compute_dtype must be torch.bfloat16 or torch.float32, not {dt}")
-        f32 = dt == torch.float32
-        if f32:
+        if dt == torch.float32:
             for name in ("cross_atten1", "cross_atten2", "cross_atten3"):
                 if any(p.dtype != torch.float32 for p in getattr(self, name).parameters()):
                     raise ValueError(f"compute_dtype float32 runs the fusion modules' fp32 engine, but {name} has been cast "
@@ -175,7 +170,7 @@ class Decoder(nn.Module):
         B = x4.shape[0]
         P = self._packed(dt)
         L = self.LEAKY
-        upcat = "cfp_upsample_concat_f32" if f32 else "cfp_upsample_concat"
+        code = _lib.dtype_code(dt)
 
         def buf(B, H, W, Cc):
             return torch.empty(B, H, W, Cc, device=dev, dtype=dt)
@@ -187,7 +182,7 @@ class Decoder(nn.Module):
                 """NCHW fp32 feature -> channels-last, channels zero-padded (cfp_upsample_concat with no low-res map)."""
                 Bq, Cq, H, W = skip.shape
                 out = buf(Bq, H, W, cpad)
-                _lib.call(upcat, 0, 1, 1, 0, 8, skip.data_ptr(), Cq, out.data_ptr(), Bq, H, W, cpad, st())
+                _lib.call("cfp_upsample_concat", 0, 1, 1, 0, 8, skip.data_ptr(), Cq, out.data_ptr(), Bq, H, W, cpad, code, st())
                 return out
 
             def up(lo, h, w, c_lo, skip, name):
@@ -195,8 +190,8 @@ class Decoder(nn.Module):
                 _, Cs, H, W = skip.shape
                 pa, pb = P[name + "a"], P[name + "b"]
                 cat = buf(B, H, W, pa.cin_pad)
-                _lib.call(upcat, lo.data_ptr(), h, w, c_lo, c_lo, skip.data_ptr(), Cs, cat.data_ptr(), B, H, W,
-                          pa.cin_pad, st())
+                _lib.call("cfp_upsample_concat", lo.data_ptr(), h, w, c_lo, c_lo, skip.data_ptr(), Cs, cat.data_ptr(), B, H, W,
+                          pa.cin_pad, code, st())
                 y = buf(B, H, W, pa.cout)
                 _conv(pa, cat, B, H, W, L, y, pa.cout, 0)
                 z = buf(B, H, W, pb.cout)
@@ -290,10 +285,8 @@ class DepthHead(nn.Module):
         dt = unet_out.dtype
         if dt == torch.float32:
             P = self._cache_f32.get(self, lambda: self._pack(dt))
-            bins, expect = "cfp_head_bins_f32", "cfp_head_expect_f32"
         elif dt == torch.bfloat16:
             P = self._cache.get(self, self._pack)
-            bins, expect = "cfp_head_bins", "cfp_head_expect"
         else:
             raise ValueError(f"unet_out must be bfloat16 (tensor-core head) or float32 (exact fp32 head), not {dt}")
         B = unet_out.shape[0]
@@ -305,14 +298,16 @@ class DepthHead(nn.Module):
         centres = torch.empty(B, nb, device=dev, dtype=torch.float32)
         pred = torch.empty(B, 1, H, W, device=dev, dtype=torch.float32)
         prob = torch.empty(B, nb, H, W, device=dev, dtype=torch.float32) if return_prob else None
+        code = _lib.dtype_code(dt)
         with torch.cuda.device(dev):
             st = _lib.stream_ptr()
             _conv(P["ram"], unet_out, B, H, W, 1.0, ram, 128, 0)
-            _lib.call(bins, unet_out.data_ptr(), 128, B, H * W, 128, P["wc"].data_ptr(), P["w0"].data_ptr(), P["b0"].data_ptr(),
-                      P["w2"].data_ptr(), P["b2"].data_ptr(), P["w4"].data_ptr(), P["b4"].data_ptr(), P["w0"].shape[0], nb,
-                      C.c_float(self.min_val), C.c_float(self.max_val), mean.data_ptr(), edges.data_ptr(), centres.data_ptr(), st)
-            _lib.call(expect, ram.data_ptr(), 128, B, H * W, P["wout"].data_ptr(), P["bout"].data_ptr(), centres.data_ptr(),
-                      nb, pred.data_ptr(), _lib.ptr(prob), st)
+            _lib.call("cfp_head_bins", unet_out.data_ptr(), 128, B, H * W, 128, P["wc"].data_ptr(), P["w0"].data_ptr(),
+                      P["b0"].data_ptr(), P["w2"].data_ptr(), P["b2"].data_ptr(), P["w4"].data_ptr(), P["b4"].data_ptr(),
+                      P["w0"].shape[0], nb, C.c_float(self.min_val), C.c_float(self.max_val), mean.data_ptr(), edges.data_ptr(),
+                      centres.data_ptr(), code, st)
+            _lib.call("cfp_head_expect", ram.data_ptr(), 128, B, H * W, P["wout"].data_ptr(), P["bout"].data_ptr(),
+                      centres.data_ptr(), nb, pred.data_ptr(), _lib.ptr(prob), code, st)
         return (edges, pred, prob) if return_prob else (edges, pred)
 
     def forward(self, unet_out: torch.Tensor):
@@ -326,6 +321,6 @@ class DepthHead(nn.Module):
             raise ValueError(f"unet_out must be bfloat16 (tensor-core head) or float32 (exact fp32 head), not {dt}")
         x = torch.empty(B, H, W, E, device=unet_out.device, dtype=dt)
         with torch.cuda.device(unet_out.device):
-            _lib.call("cfp_upsample_concat_f32" if dt == torch.float32 else "cfp_upsample_concat", 0, 1, 1, 0, 8,
-                      unet_out.detach().float().contiguous().data_ptr(), E, x.data_ptr(), B, H, W, E, _lib.stream_ptr())
+            _lib.call("cfp_upsample_concat", 0, 1, 1, 0, 8, unet_out.detach().float().contiguous().data_ptr(), E, x.data_ptr(),
+                      B, H, W, E, _lib.dtype_code(dt), _lib.stream_ptr())
         return self.forward_nhwc(x, H, W)

@@ -1,11 +1,11 @@
 """The decoder shell and adaptive-bins head in train mode (reference train.py:96-135 trains ``Deltar`` end to end with
 autograd in fp32): ``Decoder.forward`` / ``DepthHead.forward`` dispatch here when ``self.training`` is set.
 
-Every op is a libcfp kernel on fp32 channels-last maps.  The forward reuses the exact fp32 engine (``cfp_conv_f32_fwd`` with
+Every op is a libcfp kernel on fp32 channels-last maps.  The forward reuses the exact fp32 engine (``cfp_conv_fwd`` with
 the conv bias as shift and no activation, then ``cfp_tr_bn_stats`` / ``cfp_tr_bn_apply`` / LeakyReLU for a train-mode
-BatchNorm; ``cfp_upsample_concat_f32``; ``cfp_head_bins_f32`` / ``cfp_head_expect_f32``).  The backward:
+BatchNorm; ``cfp_upsample_concat``; ``cfp_head_bins`` / ``cfp_head_expect``; each with ``CFP_F32``).  The backward:
 
-* a conv's input gradient is ``cfp_conv_f32_fwd`` again, with the taps mirrored and in / out channels swapped.  That kernel
+* a conv's input gradient is ``cfp_conv_fwd`` again, with the taps mirrored and in / out channels swapped.  That kernel
   writes 32 / 64 / 128 / 256 channels per launch, so an input gradient of 80 / 168 / 232 / 312 / 392 channels is written by
   several launches into channel slices of a buffer padded to a sum of those widths (``dgrad_slices``); the pad channels have
   zero weights and every consumer reads the buffer with its pitch;
@@ -28,7 +28,7 @@ from . import _lib
 from . import train as T
 
 EW_LEAKY, EW_LEAKY_GRAD = 8, 9                 # cfp_tr_ew op codes: nn.LeakyReLU() (slope 0.01) and its gradient
-SERVED_WIDTHS = (256, 128, 64, 32)             # output channels cfp_conv_f32_fwd writes per launch
+SERVED_WIDTHS = (256, 128, 64, 32)             # output channels the fp32 cfp_conv_fwd writes per launch
 
 
 def dgrad_slices(cin: int) -> Tuple[List[Tuple[int, int]], int]:
@@ -59,7 +59,7 @@ def dgrad_weights(weight: torch.Tensor):
 
 
 def fwd_weights(weight: torch.Tensor) -> torch.Tensor:
-    """conv weight [cout, cin, k, k] -> the fp32 [k*k][cin][cout] layout of cfp_conv_f32_fwd."""
+    """conv weight [cout, cin, k, k] -> the fp32 [k*k][cin][cout] layout of cfp_conv_fwd."""
     cout, cin, k, _ = weight.shape
     return weight.detach().float().permute(2, 3, 1, 0).reshape(k * k, cin, cout).contiguous()
 
@@ -77,8 +77,8 @@ def _zeros256(dev) -> torch.Tensor:
 def conv_fwd(x: torch.Tensor, w: torch.Tensor, shift: torch.Tensor, B: int, H: int, W: int, k: int) -> torch.Tensor:
     cin, cout = w.shape[1], w.shape[2]
     out = torch.empty(B, H, W, cout, device=x.device, dtype=torch.float32)
-    _lib.call("cfp_conv_f32_fwd", x.data_ptr(), B, H, W, cin, cout, k, w.data_ptr(), shift.data_ptr(), C.c_float(1.0),
-              out.data_ptr(), cout, 0, _lib.stream_ptr())
+    _lib.call("cfp_conv_fwd", x.data_ptr(), B, H, W, cin, cout, k, 0, w.data_ptr(), shift.data_ptr(), C.c_float(1.0),
+              out.data_ptr(), cout, 0, _lib.CFP_F32, _lib.stream_ptr())
     return out
 
 
@@ -89,8 +89,8 @@ def conv_dgrad(dy: torch.Tensor, weight: torch.Tensor, B: int, H: int, W: int) -
     dx = torch.empty(B, H, W, padded, device=dy.device, dtype=torch.float32)
     zero = _zeros256(dy.device)
     for c0, w, wp in dgrad_weights(weight):
-        _lib.call("cfp_conv_f32_fwd", dy.data_ptr(), B, H, W, cout, w, k, wp.data_ptr(), zero.data_ptr(), C.c_float(1.0),
-                  dx.data_ptr(), padded, c0, _lib.stream_ptr())
+        _lib.call("cfp_conv_fwd", dy.data_ptr(), B, H, W, cout, w, k, 0, wp.data_ptr(), zero.data_ptr(), C.c_float(1.0),
+                  dx.data_ptr(), padded, c0, _lib.CFP_F32, _lib.stream_ptr())
     return dx[..., :cin]
 
 
@@ -196,8 +196,8 @@ class UpCatFn(torch.autograd.Function):
             lo_p = lo.data_ptr()
         sk = T._f32c(skip)
         out = torch.empty(B, H, W, c_lo + Cs, device=skip.device, dtype=torch.float32)
-        _lib.call("cfp_upsample_concat_f32", lo_p, h, w, c_lo, max(c_lo, 4), sk.data_ptr(), Cs, out.data_ptr(), B, H, W,
-                  c_lo + Cs, _lib.stream_ptr())
+        _lib.call("cfp_upsample_concat", lo_p, h, w, c_lo, max(c_lo, 4), sk.data_ptr(), Cs, out.data_ptr(), B, H, W,
+                  c_lo + Cs, _lib.CFP_F32, _lib.stream_ptr())
         ctx.dims = (B, h, w, c_lo, Cs, H, W)
         return out
 
@@ -214,7 +214,7 @@ class UpCatFn(torch.autograd.Function):
 
 
 class CatFn(torch.autograd.Function):
-    """torch.cat([a, b], dim=1) of decoder.py:112,117,122 on channels-last maps (cfp_copy_channels_f32 into slices)."""
+    """torch.cat([a, b], dim=1) of decoder.py:112,117,122 on channels-last maps (cfp_copy_channels into slices)."""
 
     @staticmethod
     def forward(ctx, a, b):
@@ -223,8 +223,8 @@ class CatFn(torch.autograd.Function):
         out = torch.empty(B, H, W, ca + cb, device=a.device, dtype=torch.float32)
         rows = B * H * W
         st = _lib.stream_ptr()
-        _lib.call("cfp_copy_channels_f32", a.data_ptr(), ca, out.data_ptr(), ca + cb, 0, ca, rows, st)
-        _lib.call("cfp_copy_channels_f32", T._f32c(b).data_ptr(), cb, out.data_ptr(), ca + cb, ca, cb, rows, st)
+        _lib.call("cfp_copy_channels", a.data_ptr(), ca, out.data_ptr(), ca + cb, 0, ca, rows, _lib.CFP_F32, st)
+        _lib.call("cfp_copy_channels", T._f32c(b).data_ptr(), cb, out.data_ptr(), ca + cb, ca, cb, rows, _lib.CFP_F32, st)
         ctx.ca, ctx.cb = ca, cb
         return out
 
@@ -238,8 +238,8 @@ class CatFn(torch.autograd.Function):
             st = _lib.stream_ptr()
             da = torch.empty(B, H, W, ca, device=d.device, dtype=torch.float32)
             db = torch.empty(B, H, W, cb, device=d.device, dtype=torch.float32)
-            _lib.call("cfp_copy_channels_f32", d.data_ptr(), pitch, da.data_ptr(), ca, 0, ca, rows, st)
-            _lib.call("cfp_copy_channels_f32", d.data_ptr() + 4 * ca, pitch, db.data_ptr(), cb, 0, cb, rows, st)
+            _lib.call("cfp_copy_channels", d.data_ptr(), pitch, da.data_ptr(), ca, 0, ca, rows, _lib.CFP_F32, st)
+            _lib.call("cfp_copy_channels", d.data_ptr() + 4 * ca, pitch, db.data_ptr(), cb, 0, cb, rows, _lib.CFP_F32, st)
         return da, db
 
 
@@ -324,16 +324,16 @@ class HeadFn(torch.autograd.Function):
         mean = torch.empty(B, E, device=dev, dtype=torch.float32)
         edges = torch.empty(B, nb + 1, device=dev, dtype=torch.float32)
         centres = torch.empty(B, nb, device=dev, dtype=torch.float32)
-        _lib.call("cfp_head_bins_f32", unet.data_ptr(), E, B, npix, E, wc.data_ptr(), f(reg[0].weight).data_ptr(),
+        _lib.call("cfp_head_bins", unet.data_ptr(), E, B, npix, E, wc.data_ptr(), f(reg[0].weight).data_ptr(),
                   f(reg[0].bias).data_ptr(), f(reg[2].weight).data_ptr(), f(reg[2].bias).data_ptr(), f(reg[4].weight).data_ptr(),
                   f(reg[4].bias).data_ptr(), reg[0].weight.shape[0], nb, C.c_float(head.min_val), C.c_float(head.max_val),
-                  mean.data_ptr(), edges.data_ptr(), centres.data_ptr(), st)
+                  mean.data_ptr(), edges.data_ptr(), centres.data_ptr(), _lib.CFP_F32, st)
         wout = head.conv_out[0].weight
         wout_t = wout.detach().reshape(nb, E).t().contiguous()
         pred = torch.empty(B, 1, H, W, device=dev, dtype=torch.float32)
         prob = torch.empty(B, nb, H, W, device=dev, dtype=torch.float32)
-        _lib.call("cfp_head_expect_f32", ram.data_ptr(), E, B, npix, wout_t.data_ptr(), f(head.conv_out[0].bias).data_ptr(),
-                  centres.data_ptr(), nb, pred.data_ptr(), prob.data_ptr(), st)
+        _lib.call("cfp_head_expect", ram.data_ptr(), E, B, npix, wout_t.data_ptr(), f(head.conv_out[0].bias).data_ptr(),
+                  centres.data_ptr(), nb, pred.data_ptr(), prob.data_ptr(), _lib.CFP_F32, st)
         ctx.head = head
         ctx.save_for_backward(unet, ram, mean, centres, pred, prob)
         return edges, pred

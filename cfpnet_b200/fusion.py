@@ -120,6 +120,51 @@ class TransformerFusion(nn.Module):
                 _lib.call("cfp_lkpm_fwd", feat0.data_ptr(), B, H, W, D, C.byref(lkpm_w), work.data_ptr(), ws_bytes, code, st)
         return False
 
+    def _prepare(self, x, B, H, W, feat1, kwargs, check=None):
+        """Set-up shared by ``forward`` and ``forward_tokens`` for the map ``x`` (its dtype selects the engine), in this order:
+        the shape checks, the caller's own ``check()``, the positional-encoding draws, then the packed weights, feat1 and
+        mask in the engine's types and the call's scratch.  Returns (pos, oy, ox, crop_dev, feat0, layers): ``crop_dev`` is
+        the device crop buffer under a CUDA-graph capture (oy = ox = 0 then), else None; ``feat0`` is the [B, H*W, D] token
+        map the caller fills; ``layers(st, out_nchw=None)`` runs the layer list on it (``_run_layers``)."""
+        D, dt, dev = self.embedding_dim, x.dtype, x.device
+        S = feat1.size(2)
+        g = zone_geometry(kwargs["patch_info"], self.max_resolution[1], H, W)
+        if any(n in ("hist2image", "combine1") for n in self.layer_names):
+            check_geometry(g, H, W)
+        if feat1.shape[0] != B or feat1.shape[1] != g.zone_num ** 2 or feat1.shape[3] != D:
+            raise ValueError(f"feat1 {tuple(feat1.shape)} does not match B={B}, zones={g.zone_num ** 2}, D={D}")
+        if S != self.positional_encodings2.shape[0]:     # the reference's `feat1 + positional_encodings2` fails to broadcast
+            raise ValueError(f"feat1 carries {S} samples per zone, positional_encodings2 has {self.positional_encodings2.shape[0]}")
+        if tuple(kwargs["mask"].shape) != (B, g.zone_num ** 2):
+            raise ValueError(f"mask {tuple(kwargs['mask'].shape)} is not [B={B}, zones={g.zone_num ** 2}]")
+        if check is not None:
+            check()
+
+        # positional-encoding crop: same draws, same order as fusion.py:87-91 (under a CUDA-graph capture the offsets live
+        # in device memory and the replay wrapper makes the draws: FusionPath.make_graphed, pipeline.make_graphed_depth)
+        crop_dev = self.__dict__.get("_crop_dev")
+        oy, ox = (0, 0) if crop_dev is not None else self.draw_crop(H, W)
+
+        packed, pos, pos2, _buf = self._cache.get(self, self._pack)
+        feat1 = feat1.detach().to(dt).contiguous()
+        mask = kwargs["mask"].to(device=dev, dtype=torch.uint8).contiguous()
+        cg = _lib.CfpGeom.from_geometry(g)
+        emb_copy = (not args.change_embedding) and "hist2image" in self.layer_names
+        code = _lib.dtype_code(dt)
+        ws_bytes = _lib.load().cfp_workspace_bytes(B, H, W, D, self.ws, self.large_kernel or 0, code, C.byref(cg))
+        # scratch (workspace + token map) is owned by the module and reused across calls: stream order
+        # makes that safe for back-to-back forwards on one stream, and it keeps hundreds of MB of
+        # per-call allocations (cudaMalloc stalls once several streams are in play) off the hot path.
+        # One module instance must not run on two streams at once (replicas own their scratch).
+        work, feat0 = self._scratch.get(
+            dev.index, (dt, B, H, W), lambda t: t[0].numel() >= ws_bytes,
+            lambda: (torch.empty(ws_bytes, device=dev, dtype=torch.uint8), torch.empty(B, H * W, D, device=dev, dtype=dt)))
+
+        def layers(st, out_nchw=None):
+            return self._run_layers(packed, pos2, feat0, feat1, mask, B, H, W, D, S, cg, work, ws_bytes, code, st, emb_copy,
+                                    out_nchw=out_nchw)
+        return pos, oy, ox, crop_dev, feat0, layers
+
     def forward_tokens(self, x_tok, x_pitch, B, H, W, feat1, out_tok, out_pitch, out_coff, **kwargs):
         """The same call for a caller that holds its maps channels-last (cfpnet_b200.decoder): ``x_tok`` is a
         [B, H, W, x_pitch] buffer whose first ``embedding_dim`` channels are x; the result is written into channels
@@ -133,45 +178,14 @@ class TransformerFusion(nn.Module):
         dt = x_tok.dtype
         if dt not in (torch.bfloat16, torch.float32) or out_tok.dtype != dt:
             raise ValueError(f"forward_tokens needs x_tok and out_tok both bf16 or both fp32 (got {x_tok.dtype} and {out_tok.dtype})")
-        S = feat1.size(2)
-        g = zone_geometry(kwargs["patch_info"], self.max_resolution[1], H, W)
-        if any(n in ("hist2image", "combine1") for n in self.layer_names):
-            check_geometry(g, H, W)
-        if feat1.shape[0] != B or feat1.shape[1] != g.zone_num ** 2 or feat1.shape[3] != D:
-            raise ValueError(f"feat1 {tuple(feat1.shape)} does not match B={B}, zones={g.zone_num ** 2}, D={D}")
-        if S != self.positional_encodings2.shape[0]:
-            raise ValueError(f"feat1 carries {S} samples per zone, positional_encodings2 has {self.positional_encodings2.shape[0]}")
-        if tuple(kwargs["mask"].shape) != (B, g.zone_num ** 2):
-            raise ValueError(f"mask {tuple(kwargs['mask'].shape)} is not [B={B}, zones={g.zone_num ** 2}]")
-        # under a CUDA-graph capture the crop offsets live in device memory and the replay wrapper makes the draws
-        # (cfpnet_b200.pipeline.make_graphed_depth), as in forward()
-        crop_dev = self.__dict__.get("_crop_dev")
-        oy, ox = (0, 0) if crop_dev is not None else self.draw_crop(H, W)
-        packed, pos, pos2, _buf = self._cache.get(self, self._pack)
-        dev = x_tok.device
+        pos, oy, ox, crop_dev, feat0, layers = self._prepare(x_tok, B, H, W, feat1, kwargs)
         code = _lib.dtype_code(dt)
-        posenc, posenc_crop, copy = (
-            ("cfp_posenc_tokens_nhwc_f32_fwd", "cfp_posenc_tokens_nhwc_f32_crop_fwd", "cfp_copy_channels_f32") if dt == torch.float32
-            else ("cfp_posenc_tokens_nhwc_fwd", "cfp_posenc_tokens_nhwc_crop_fwd", "cfp_copy_channels"))
-        feat1 = feat1.detach().to(dt).contiguous()
-        mask = kwargs["mask"].to(device=dev, dtype=torch.uint8).contiguous()
-        cg = _lib.CfpGeom.from_geometry(g)
-        emb_copy = (not args.change_embedding) and "hist2image" in self.layer_names
-        with torch.cuda.device(dev):
-            lib = _lib.load()
-            ws_bytes = lib.cfp_workspace_bytes(B, H, W, D, self.ws, self.large_kernel or 0, code, C.byref(cg))
-            work, feat0 = self._scratch.get(
-                dev.index, (dt, B, H, W), lambda t: t[0].numel() >= ws_bytes,
-                lambda: (torch.empty(ws_bytes, device=dev, dtype=torch.uint8), torch.empty(B, H * W, D, device=dev, dtype=dt)))
+        with torch.cuda.device(x_tok.device):
             st = _lib.stream_ptr()
-            if crop_dev is not None:
-                _lib.call(posenc_crop, x_tok.data_ptr(), x_pitch, pos, feat0.data_ptr(), B, D, H, W,
-                          self.max_resolution[0], self.max_resolution[1], crop_dev.data_ptr(), st)
-            else:
-                _lib.call(posenc, x_tok.data_ptr(), x_pitch, pos, feat0.data_ptr(), B, D, H, W,
-                          self.max_resolution[0], self.max_resolution[1], oy, ox, st)
-            self._run_layers(packed, pos2, feat0, feat1, mask, B, H, W, D, S, cg, work, ws_bytes, code, st, emb_copy)
-            _lib.call(copy, feat0.data_ptr(), D, out_tok.data_ptr(), out_pitch, out_coff, D, B * H * W, st)
+            _lib.call("cfp_posenc_tokens_nhwc_fwd", x_tok.data_ptr(), x_pitch, pos, feat0.data_ptr(), B, D, H, W,
+                      self.max_resolution[0], self.max_resolution[1], oy, ox, _lib.ptr(crop_dev), code, st)
+            layers(st)
+            _lib.call("cfp_copy_channels", feat0.data_ptr(), D, out_tok.data_ptr(), out_pitch, out_coff, D, B * H * W, code, st)
         return out_tok
 
     # ------------------------------------------------------------------ forward
@@ -217,59 +231,26 @@ class TransformerFusion(nn.Module):
             raise ValueError(f"x has {D} channels, module was built for {self.embedding_dim}")
         dt = x.dtype
         code = _lib.dtype_code(dt)
-        S = feat1.size(2)
-        g = zone_geometry(kwargs["patch_info"], self.max_resolution[1], H, W)
-        uses_zones = any(n in ("hist2image", "combine1") for n in self.layer_names)
-        if uses_zones:
-            check_geometry(g, H, W)
-        if feat1.shape[0] != B or feat1.shape[1] != g.zone_num ** 2 or feat1.shape[3] != D:
-            raise ValueError(f"feat1 {tuple(feat1.shape)} does not match B={B}, zones={g.zone_num ** 2}, D={D}")
-        if S != self.positional_encodings2.shape[0]:     # the reference's `feat1 + positional_encodings2` fails to broadcast
-            raise ValueError(f"feat1 carries {S} samples per zone, positional_encodings2 has {self.positional_encodings2.shape[0]}")
-        if tuple(kwargs["mask"].shape) != (B, g.zone_num ** 2):
-            raise ValueError(f"mask {tuple(kwargs['mask'].shape)} is not [B={B}, zones={g.zone_num ** 2}]")
-        if torch.is_grad_enabled() and (x.requires_grad or feat1.requires_grad):
-            raise RuntimeError("TransformerFusion (libcfp, eval mode) returns a tensor without autograd history: an input "
-                               "that requires grad would have its gradient cut silently; call under torch.no_grad() or "
-                               "detach the inputs")
 
-        # positional-encoding crop: same draws, same order as fusion.py:87-91 (under a CUDA-graph capture the offsets
-        # live in device memory and the replay wrapper makes the draws: FusionPath.make_graphed)
-        crop_dev = self.__dict__.get("_crop_dev")
-        oy, ox = (0, 0) if crop_dev is not None else self.draw_crop(H, W)
+        def refuse_grad():
+            if torch.is_grad_enabled() and (x.requires_grad or feat1.requires_grad):
+                raise RuntimeError("TransformerFusion (libcfp, eval mode) returns a tensor without autograd history: an input "
+                                   "that requires grad would have its gradient cut silently; call under torch.no_grad() or "
+                                   "detach the inputs")
 
-        packed, pos, pos2, _buf = self._cache.get(self, self._pack)
+        pos, oy, ox, crop_dev, feat0, layers = self._prepare(x, B, H, W, feat1, kwargs, check=refuse_grad)
         dev = x.device
         x = x.detach().contiguous()
-        feat1 = feat1.detach().to(dt).contiguous()
-        mask = kwargs["mask"].to(device=dev, dtype=torch.uint8).contiguous()
-        cg = _lib.CfpGeom.from_geometry(g)
         out = kwargs.get("out")                  # optional caller-provided result buffer (same shape/dtype)
         if out is None:
             out = torch.empty(B, D, H, W, device=dev, dtype=dt)
         elif out.shape != x.shape or out.dtype != dt or out.device != dev or not out.is_contiguous():
             raise ValueError("out= must be a contiguous tensor shaped and typed like x")
-        emb_copy = (not args.change_embedding) and "hist2image" in self.layer_names
 
         with torch.cuda.device(dev):
-            lib = _lib.load()
-            ws_bytes = lib.cfp_workspace_bytes(B, H, W, D, self.ws, self.large_kernel or 0, code, C.byref(cg))
-            # scratch (workspace + token map) is owned by the module and reused across calls: stream order
-            # makes that safe for back-to-back forwards on one stream, and it keeps hundreds of MB of
-            # per-call allocations (cudaMalloc stalls once several streams are in play) off the hot path.
-            # One module instance must not run on two streams at once (replicas own their scratch).
-            work, feat0 = self._scratch.get(
-                dev.index, (dt, B, H, W), lambda t: t[0].numel() >= ws_bytes,
-                lambda: (torch.empty(ws_bytes, device=dev, dtype=torch.uint8),
-                         torch.empty(B, H * W, D, device=dev, dtype=dt)))
             st = _lib.stream_ptr()
-            if crop_dev is not None:
-                _lib.call("cfp_posenc_tokens_crop_fwd", x.data_ptr(), pos, feat0.data_ptr(), B, D, H, W,
-                          self.max_resolution[0], self.max_resolution[1], crop_dev.data_ptr(), code, st)
-            else:
-                _lib.call("cfp_posenc_tokens_fwd", x.data_ptr(), pos, feat0.data_ptr(), B, D, H, W,
-                          self.max_resolution[0], self.max_resolution[1], oy, ox, code, st)
-            if not self._run_layers(packed, pos2, feat0, feat1, mask, B, H, W, D, S, cg, work, ws_bytes, code, st, emb_copy,
-                                    out_nchw=out):
+            _lib.call("cfp_posenc_tokens_fwd", x.data_ptr(), pos, feat0.data_ptr(), B, D, H, W,
+                      self.max_resolution[0], self.max_resolution[1], oy, ox, _lib.ptr(crop_dev), code, st)
+            if not layers(st, out_nchw=out):
                 _lib.call("cfp_tokens_to_nchw", feat0.data_ptr(), out.data_ptr(), B, D, H, W, code, st)
         return out

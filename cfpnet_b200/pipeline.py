@@ -126,8 +126,8 @@ class FusionPath(nn.Module):
         inputs (``run()`` takes no arguments; the caller refills them in place).
 
         The positional-encoding crop offsets (``fusion.py:88-91``, drawn per forward when a map is smaller than its
-        table) are not frozen into the graph: while capturing, the modules read them from a small device buffer
-        (``cfp_posenc_tokens_crop_fwd``), and every replay first makes the reference's draws - same generator, same
+        table) are not frozen into the graph: while capturing, the modules read them from a small device buffer (the crop
+        pointer of ``cfp_posenc_tokens_fwd``), and every replay first makes the reference's draws - same generator, same
         order L3, L2, L1 - and uploads them."""
         mods = ((self.cross_atten3, x3), (self.cross_atten2, x2), (self.cross_atten1, x1))
         static = [t.clone() for t in (x3, x2, x1, hist_data, mask)] if copy_inputs else [x3, x2, x1, hist_data, mask]
@@ -366,9 +366,9 @@ def make_graphed_depth(hist_encoder: HistogramEncoder, decoder, head, img_featur
     ``args.change_embedding`` it was captured with.
 
     Positional-encoding crops are not frozen: while capturing, the fusion modules read their offsets from a device buffer
-    (``cfp_posenc_tokens_nhwc_crop_fwd``), and every replay first makes the reference's draws from torch's global generator
-    in the decoder's order (``cross_atten3``, ``2``, ``1``; oy then ox; nothing drawn along an axis the map fills) and
-    uploads them with a stream-ordered copy, so the generator advances exactly as in an eager forward.
+    (the crop pointer of ``cfp_posenc_tokens_nhwc_fwd``), and every replay first makes the reference's draws from torch's
+    global generator in the decoder's order (``cross_atten3``, ``2``, ``1``; oy then ox; nothing drawn along an axis the map
+    fills) and uploads them with a stream-ordered copy, so the generator advances exactly as in an eager forward.
 
     Ownership and staleness: ``run`` keeps the fusion modules' scratch tensors and every packed-weight copy the graph reads
     alive, so an eager call at another shape or a re-pack cannot free memory under it.  ``run`` raises ``CfpError`` instead

@@ -274,7 +274,7 @@ def _nchw_to_tokens(x: torch.Tensor) -> torch.Tensor:
     B, Cc, H, W = x.shape
     tok = torch.empty(B * H * W, Cc, device=x.device, dtype=torch.float32)
     zero_pos = torch.zeros(H * W, Cc, device=x.device, dtype=torch.float32)
-    _lib.call("cfp_posenc_tokens_fwd", x.data_ptr(), zero_pos.data_ptr(), tok.data_ptr(), B, Cc, H, W, H, W, 0, 0,
+    _lib.call("cfp_posenc_tokens_fwd", x.data_ptr(), zero_pos.data_ptr(), tok.data_ptr(), B, Cc, H, W, H, W, 0, 0, None,
               _lib.CFP_F32, _st())
     return tok
 
@@ -419,7 +419,7 @@ class CudaOps:
         B, Cc, H, W = x.shape
         tok = torch.empty(B * H * W, Cc, device=x.device, dtype=torch.float32)
         _lib.call("cfp_posenc_tokens_fwd", _f32c(x).data_ptr(), _f32c(pos).data_ptr(), tok.data_ptr(), B, Cc, H, W,
-                  int(max_res[0]), int(max_res[1]), int(oy), int(ox), _lib.CFP_F32, _st())
+                  int(max_res[0]), int(max_res[1]), int(oy), int(ox), None, _lib.CFP_F32, _st())
         return tok
 
     def nchw_to_tokens(self, x):

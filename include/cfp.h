@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define CFP_ABI_VERSION 15
+#define CFP_ABI_VERSION 16
 
 #if defined(__GNUC__)
 #define CFP_API __attribute__((visibility("default")))
@@ -158,15 +158,15 @@ CFP_API int cfp_zone_masks(const uint8_t *mask, uint8_t *zone_mask, uint8_t *his
 
 /* a4. Positional-encoding add + NCHW -> token-major (fusion.py:92-97):
  * tokens[b][y*W+x][c] = x[b][c][y][x] + pos[(oy+y)*pos_w + ox+x][c]; pos is the
- * [pos_h*pos_w][C] table (max_resolution), the crop must lie inside it. */
+ * [pos_h*pos_w][C] table (max_resolution).  The crop offsets come from one of two places:
+ *   crop == NULL: (oy, ox) as passed; the crop must lie inside the table.
+ *   crop != NULL: (oy, ox) = (crop[0], crop[1]), int32 in DEVICE memory, read when the kernel runs: a CUDA-graph replay of
+ *     a forward then takes fresh offsets from the buffer instead of freezing the captured ones (the reference draws them
+ *     per call, fusion.py:88-91).  The host cannot see these offsets and does not range-check them: the caller keeps
+ *     0 <= crop[0] <= pos_h - H, 0 <= crop[1] <= pos_w - W.  The map must fit the table, and oy, ox must be 0. */
 CFP_API int cfp_posenc_tokens_fwd(const void *x_nchw, const float *pos, void *tokens, int B, int C, int H,
-                          int W, int pos_h, int pos_w, int oy, int ox, int dtype, void *stream);
+                          int W, int pos_h, int pos_w, int oy, int ox, const int *crop, int dtype, void *stream);
 /* fusion.py:186: token-major -> contiguous NCHW. */
-/* cfp_posenc_tokens_fwd with the crop offsets (oy, ox) read from DEVICE memory (crop [2], int32) when the kernel runs: a
- * CUDA-graph replay of a forward then takes fresh offsets from the buffer instead of freezing the captured ones (the
- * reference draws them per call, fusion.py:88-91).  The caller keeps 0 <= oy <= pos_h - H, 0 <= ox <= pos_w - W. */
-CFP_API int cfp_posenc_tokens_crop_fwd(const void *x_nchw, const float *pos, void *tokens, int B, int C, int H, int W, int pos_h,
-                                       int pos_w, const int *crop, int dtype, void *stream);
 CFP_API int cfp_tokens_to_nchw(const void *tokens, void *out_nchw, int B, int C, int H, int W, int dtype,
                        void *stream);
 
@@ -285,91 +285,71 @@ CFP_API int cfp_tr_adamw(float *p, const float *g, float *m, float *v, int64_t n
                          int nseg, float beta1, float beta2, float eps, float weight_decay, int step, float grad_scale,
                          const float *sumsq, float max_norm, void *stream);
 
-/* ---- Decoder shell (SURVEY.md 8 f1) and adaptive-bins head (f2): bf16, channels-last maps [B][H][W][pitch] - the token-major
- * layout of the fusion path.
+/* ---- Decoder shell (SURVEY.md 8 f1) and adaptive-bins head (f2) on channels-last maps [B][H][W][pitch] - the token-major
+ * layout of the fusion path.  `dtype` selects the engine and the element type of the maps:
+ *   CFP_BF16: bf16 maps, the convolutions and conv_out on the tensor cores (tcgen05); the channel counts, pitches and
+ *     channel offsets of the channels-last maps are multiples of 8;
+ *   CFP_F32: the exact fp32 engine: fp32 maps, fp32 FFMA with fp32 accumulation (no TF32 or bf16 operands), no atomics
+ *     (every output is summed in one fixed order: two runs give the same bits); those counts are multiples of 4.
  *
- * cfp_conv_fwd: k x k convolution (k = 1, 3; stride 1, zero padding (k-1)/2) as an implicit GEMM on tcgen05:
+ * cfp_conv_fwd: k x k convolution (k = 1, 3; stride 1, zero padding (k-1)/2) as an implicit GEMM:
  *   out[b][y][x][out_coff + o] = act(sum_{taps, c} in[b][y+dy][x+dx][c] w[o][c][dy][dx] + shift[o]), act = LeakyReLU with
  *   `leaky_slope` (1.0 = none).  Serves decoder.py:43-48 (conv3x3 + BatchNorm2d folded by the host + LeakyReLU, twice per
- *   UpSampleBN), :70,76-80 (1x1 / 3x3 convs with bias) and DepthRegression.conv3x3 (:13).  cin: input channels, zero-padded to
- *   a multiple of 16 (= the input's pitch); cout in {32, 64, 128, 256}; kchunk (multiple of 16, divides cin, cout * kchunk <=
- *   20480): channels per staged K-chunk; w_tc: bf16 blocks [cin / kchunk][k * k][kchunk / 8][cout][8] (canonical K-major UMMA
- *   layout per (chunk, tap)); shift [cout] fp32; out: bf16, pitch out_pitch (write into a slice of a wider buffer: torch.cat).
+ *   UpSampleBN), :70,76-80 (1x1 / 3x3 convs with bias) and DepthRegression.conv3x3 (:13).  cout in {32, 64, 128, 256};
+ *   shift [cout] fp32; out has pitch out_pitch (write into a slice of a wider buffer: torch.cat).
+ *   CFP_BF16: cin: input channels, zero-padded to a multiple of 16 (= the input's pitch); kchunk (multiple of 16, divides
+ *     cin, cout * kchunk <= 20480): channels per staged K-chunk; w: bf16 blocks [cin / kchunk][k * k][kchunk / 8][cout][8]
+ *     (canonical K-major UMMA layout per (chunk, tap)).
+ *   CFP_F32: cin is a multiple of 4 and equal to the input's pitch (no padding); kchunk must be 0 (no K-chunks); w is fp32
+ *     [k * k][cin][cout] (tap = ky * k + kx).
  * cfp_upsample_concat: UpSampleBN's input (decoder.py:51-58): out [B][H][W][c_out] = [ bilinear(align_corners) resize of
- *   lo [B][h][w][c_lo] (pitch lo_pitch) | skip [B][c_skip][H][W] (fp32 NCHW, the image encoder's feature) | zeros ].
- * cfp_copy_channels: dst[row][coff : coff + C] = src[row][0 : C] (bf16, pitches in elements).
+ *   lo [B][h][w][c_lo] (pitch lo_pitch) | skip [B][c_skip][H][W] (fp32 NCHW, the image encoder's feature; any c_skip) | zeros ].
+ * cfp_posenc_tokens_nhwc_fwd: cfp_posenc_tokens_fwd for a caller that already holds the map channels-last (pitch x_pitch):
+ *   tokens = x + pos crop, with the same two sources of the crop offsets (crop == NULL: oy, ox, range-checked; crop !=
+ *   NULL: device offsets the caller keeps inside the table, oy = ox = 0): a CUDA-graph replay of the decoder takes fresh
+ *   offsets from the buffer.
+ * cfp_copy_channels: dst[row][coff : coff + C] = src[row][0 : C] (pitches in elements).
  * cfp_head_bins: DepthRegression's regressor branch (decoder.py:24-36, norm 'linear') + the bin geometry of deltar.py:52-57:
  *   per-frame channel mean of x [B][npix][pitch] (E channels) -> conv1x1 (wc [E][E], no bias) -> Linear(E, hidden) ->
  *   LeakyReLU -> Linear(hidden, hidden) -> LeakyReLU -> Linear(hidden, n_bins) -> relu + 0.1 -> / sum -> edges [B][n_bins + 1]
  *   = cumsum([min_val, (max_val - min_val) y]), centres [B][n_bins].  Weights fp32 row-major [out][in]; mean_scratch [B][E].
+ *   CFP_F32 forms the channel mean per frame in one CTA (no atomics); the regressor is the same for both engines.
  * cfp_head_expect: conv_out (1x1, E = 128 -> n_bins, bias) + softmax over the bins + sum_j p_j centre_j in one kernel:
- *   x [B][npix][pitch] bf16 (the range-attention maps), w_tc = canonical UMMA block of the [n_bins][128] weight, pred
- *   [B][npix] fp32; prob (nullable) [B][n_bins][npix] fp32 is the probability volume the reference returns in eval mode. */
-CFP_API int cfp_conv_fwd(const void *in, int B, int H, int W, int cin, int cout, int ksize, int kchunk, const void *w_tc,
-                         const float *shift, float leaky_slope, void *out, int out_pitch, int out_coff, void *stream);
+ *   x [B][npix][pitch] (the range-attention maps), pred [B][npix] fp32; prob (nullable) [B][n_bins][npix] fp32 is the
+ *   probability volume the reference returns in eval mode.  w is conv_out's [n_bins][128] weight: for CFP_BF16 the
+ *   canonical UMMA block, for CFP_F32 transposed to fp32 [128][n_bins] (softmax with expf and true divisions). */
+CFP_API int cfp_conv_fwd(const void *in, int B, int H, int W, int cin, int cout, int ksize, int kchunk, const void *w,
+                         const float *shift, float leaky_slope, void *out, int out_pitch, int out_coff, int dtype, void *stream);
 CFP_API int cfp_upsample_concat(const void *lo, int h, int w, int c_lo, int lo_pitch, const float *skip, int c_skip, void *out,
-                                int B, int H, int W, int c_out, void *stream);
-/* cfp_posenc_tokens_fwd for a caller that already holds the map channels-last (bf16, pitch x_pitch): tokens = x + pos crop. */
+                                int B, int H, int W, int c_out, int dtype, void *stream);
 CFP_API int cfp_posenc_tokens_nhwc_fwd(const void *x, int x_pitch, const float *pos, void *tokens, int B, int C, int H, int W,
-                                       int pos_h, int pos_w, int oy, int ox, void *stream);
-/* cfp_posenc_tokens_nhwc_fwd with the crop offsets (oy, ox) read from DEVICE memory (crop [2], int32) when the kernel runs, as
- * cfp_posenc_tokens_crop_fwd: a CUDA-graph replay of the decoder takes fresh offsets from the buffer.  The host cannot see the
- * offsets and does not range-check them: the caller keeps 0 <= oy <= pos_h - H, 0 <= ox <= pos_w - W. */
-CFP_API int cfp_posenc_tokens_nhwc_crop_fwd(const void *x, int x_pitch, const float *pos, void *tokens, int B, int C, int H, int W,
-                                            int pos_h, int pos_w, const int *crop, void *stream);
-CFP_API int cfp_copy_channels(const void *src, int src_pitch, void *dst, int dst_pitch, int coff, int C, int64_t rows, void *stream);
+                                       int pos_h, int pos_w, int oy, int ox, const int *crop, int dtype, void *stream);
+CFP_API int cfp_copy_channels(const void *src, int src_pitch, void *dst, int dst_pitch, int coff, int C, int64_t rows, int dtype,
+                              void *stream);
 CFP_API int cfp_head_bins(const void *x, int pitch, int B, int npix, int E, const float *wc, const float *w0, const float *b0,
                           const float *w2, const float *b2, const float *w4, const float *b4, int hidden, int n_bins, float min_val,
-                          float max_val, float *mean_scratch, float *edges, float *centres, void *stream);
-CFP_API int cfp_head_expect(const void *x, int pitch, int B, int npix, const void *w_tc, const float *bias, const float *centres,
-                            int n_bins, float *pred, float *prob, void *stream);
-
-/* ---- The same stages on the exact fp32 engine: fp32 channels-last maps, fp32 FFMA with fp32 accumulation (no TF32 or bf16
- * operands), no atomics (every output is summed in one fixed order: two runs give the same bits).  Each call has the
- * contract of its bf16 sibling above, except:
- * cfp_conv_f32_fwd: cin is a multiple of 4 and equal to the input's pitch (no padding, no K-chunk argument); w is fp32
- *   [k * k][cin][cout] (tap = ky * k + kx); out_pitch and out_coff are multiples of 4.
- * cfp_upsample_concat_f32, cfp_copy_channels_f32, cfp_posenc_tokens_nhwc_f32_fwd: channel counts, pitches and offsets are
- *   multiples of 4.
- * cfp_head_bins_f32: x is fp32; the channel mean is formed per frame in one CTA (no atomics), then the regressor of
- *   cfp_head_bins.
- * cfp_head_expect_f32: x fp32 [B][npix][pitch]; w_t = conv_out's weight as fp32 [128][n_bins]; softmax with expf and true
- *   divisions. */
-CFP_API int cfp_conv_f32_fwd(const float *in, int B, int H, int W, int cin, int cout, int ksize, const float *w, const float *shift,
-                             float leaky_slope, float *out, int out_pitch, int out_coff, void *stream);
-CFP_API int cfp_upsample_concat_f32(const float *lo, int h, int w, int c_lo, int lo_pitch, const float *skip, int c_skip, float *out,
-                                    int B, int H, int W, int c_out, void *stream);
-CFP_API int cfp_posenc_tokens_nhwc_f32_fwd(const float *x, int x_pitch, const float *pos, float *tokens, int B, int C, int H, int W,
-                                           int pos_h, int pos_w, int oy, int ox, void *stream);
-/* The fp32 form of cfp_posenc_tokens_nhwc_crop_fwd (same contract: the caller keeps the crop inside the table). */
-CFP_API int cfp_posenc_tokens_nhwc_f32_crop_fwd(const float *x, int x_pitch, const float *pos, float *tokens, int B, int C, int H,
-                                                int W, int pos_h, int pos_w, const int *crop, void *stream);
-CFP_API int cfp_copy_channels_f32(const float *src, int src_pitch, float *dst, int dst_pitch, int coff, int C, int64_t rows,
-                                  void *stream);
-CFP_API int cfp_head_bins_f32(const float *x, int pitch, int B, int npix, int E, const float *wc, const float *w0, const float *b0,
-                              const float *w2, const float *b2, const float *w4, const float *b4, int hidden, int n_bins,
-                              float min_val, float max_val, float *mean_scratch, float *edges, float *centres, void *stream);
-CFP_API int cfp_head_expect_f32(const float *x, int pitch, int B, int npix, const float *w_t, const float *bias, const float *centres,
-                                int n_bins, float *pred, float *prob, void *stream);
+                          float max_val, float *mean_scratch, float *edges, float *centres, int dtype, void *stream);
+CFP_API int cfp_head_expect(const void *x, int pitch, int B, int npix, const void *w, const float *bias, const float *centres,
+                            int n_bins, float *pred, float *prob, int dtype, void *stream);
 
 /* ---- The decoder shell and head in train mode (reference train.py:96-135 differentiates decoder.py / deltar.py:50-61 with
  * autograd): the adjoints no forward kernel computes.  fp32 FFMA, no atomics, fixed summation order (two launches give the
- * same bits).  cfpnet_b200/decoder_train.py sequences them with the forward kernels above: a conv's input gradient is
- * cfp_conv_f32_fwd with the taps mirrored and in / out channels swapped.
+ * same bits).  cfpnet_b200/decoder_train.py sequences them with the forward kernels above on the CFP_F32 engine: a conv's
+ * input gradient is cfp_conv_fwd with the taps mirrored and in / out channels swapped.
  *
  * cfp_tr_conv_wgrad_f32: weight gradient of a k x k conv (k = 1, 3; stride 1, zero padding k / 2) on channels-last maps,
  *   dw[tap][ci][co] = sum_{b,y,x} x[b][y + ky - k/2][x + kx - k/2][ci] dy[b][y][x][co] (tap = ky k + kx: the fp32 weight
- *   layout of cfp_conv_f32_fwd).  cin, cout multiples of 4; x has pitch cin, dy pitch cout.  The B*H*W pixels are split
+ *   layout of cfp_conv_fwd with CFP_F32).  cin, cout multiples of 4; x has pitch cin, dy pitch cout.  The B*H*W pixels are split
  *   into ranges, each writes a partial into `scratch`, a second pass adds them in range order:
  *   cfp_tr_conv_wgrad_scratch_floats(B, H, W, cin, cout, ksize) floats (pure host arithmetic; 0 = no scratch needed).
- * cfp_tr_upsample_concat_bwd_f32: adjoint of cfp_upsample_concat_f32.  dcat [B][H][W][pitch] -> d_lo [B][h][w][c_lo]
+ * cfp_tr_upsample_concat_bwd_f32: adjoint of cfp_upsample_concat with CFP_F32.  dcat [B][H][W][pitch] -> d_lo [B][h][w][c_lo]
  *   (channels-last, the adjoint of the align_corners bilinear resize, gathered per low-resolution pixel) and d_skip
  *   [B][c_skip][H][W] (NCHW, channels c_lo .. c_lo + c_skip of dcat).
- * cfp_tr_head_expect_bwd_f32: adjoint of cfp_head_expect_f32 given its probability volume prob [B][n_bins][npix], pred
+ * cfp_tr_head_expect_bwd_f32: adjoint of cfp_head_expect with CFP_F32 given its probability volume prob [B][n_bins][npix], pred
  *   [B][npix], centres [B][n_bins] and dpred [B][npix]: dlogit [B*npix][n_bins] = p (centre - pred) dpred, dcentres
  *   [B][n_bins] = sum_pixels p dpred.  scratch: B * ((npix + 31) / 32) * n_bins floats.
  * cfp_tr_head_bins_bwd_f32: one CTA per frame.  z [B][n_bins] = the regressor's output before relu + 0.1; d_edges [B][n_bins
- *   + 1] and d_centres [B][n_bins] (either nullable = zero) are the cotangents of cfp_head_bins_f32's outputs -> dz. */
+ *   + 1] and d_centres [B][n_bins] (either nullable = zero) are the cotangents of cfp_head_bins's outputs -> dz. */
 CFP_API size_t cfp_tr_conv_wgrad_scratch_floats(int B, int H, int W, int cin, int cout, int ksize);
 CFP_API int cfp_tr_conv_wgrad_f32(const float *x, const float *dy, float *dw, float *scratch, int B, int H, int W, int cin, int cout,
                                   int ksize, void *stream);

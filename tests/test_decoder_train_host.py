@@ -1,5 +1,5 @@
 """CPU checks of the decoder shell / head training path's host arithmetic: the input-gradient weight packing and channel-slice
-plan (applied by a restatement of what cfp_conv_f32_fwd computes per tap) against torch's conv2d_input, the gather ranges
+plan (applied by a restatement of what the fp32 cfp_conv_fwd computes per tap) against torch's conv2d_input, the gather ranges
 and weights of the upsample adjoint (restated in fp32 as cfp_tr_upsample_concat_bwd_f32 forms them) against autograd of
 F.interpolate, the train-mode fp64 reference of UpSampleBN the GPU tests compare against, and the weight-gradient scratch
 size (pure host arithmetic).  No device work."""
@@ -22,7 +22,7 @@ CONV_SHAPES = [(232, 256, 1), (392, 256, 3), (256, 256, 3), (256, 128, 1), (312,
 
 
 def conv_f32_restated(x_nhwc, w, out, out_coff):
-    """What cfp_conv_f32_fwd computes (zero shift, slope 1): out[..., coff + o] = sum_{tap, c} x[p + off(tap)][c] w[tap][c][o]."""
+    """What the fp32 cfp_conv_fwd computes (zero shift, slope 1): out[..., coff + o] = sum_{tap, c} x[p + off(tap)][c] w[tap][c][o]."""
     B, H, W, _ = x_nhwc.shape
     taps, _, n = w.shape
     k = int(round(math.sqrt(taps)))

@@ -1,4 +1,4 @@
-"""Host side of the whole-model CUDA graph (no GPU needed): argument checks of the NHWC positional-encoding entry points with
+"""Host side of the whole-model CUDA graph (no GPU needed): argument checks of the NHWC positional-encoding entry point with
 device-resident crop offsets, and the capture guard of cfpnet_b200.pipeline.make_graphed_depth on CPU modules."""
 import pytest
 import torch
@@ -8,22 +8,23 @@ from cfpnet_b200 import _lib, decoder as D, synth
 from cfpnet_b200.config import args
 from cfpnet_b200.pipeline import _CaptureGuard
 
-CROP_ENTRIES = ("cfp_posenc_tokens_nhwc_crop_fwd", "cfp_posenc_tokens_nhwc_f32_crop_fwd")
 FAKE = 256                      # a non-null "device pointer": every call below is refused before anything is launched
 
 
-@pytest.mark.parametrize("name", CROP_ENTRIES)
-def test_crop_entry_points_refuse_bad_arguments(name):
-    ok = dict(x=FAKE, pitch=128, pos=FAKE, tok=FAKE, B=1, C=64, H=26, W=34, ph=30, pw=40, crop=FAKE)
+@pytest.mark.parametrize("dtype", [_lib.CFP_BF16, _lib.CFP_F32], ids=["bf16", "f32"])
+def test_crop_entry_points_refuse_bad_arguments(dtype):
+    ok = dict(x=FAKE, pitch=128, pos=FAKE, tok=FAKE, B=1, C=64, H=26, W=34, ph=30, pw=40, oy=0, ox=0, crop=FAKE, dtype=dtype)
 
     def call(**kw):
         a = {**ok, **kw}
-        _lib.call(name, a["x"], a["pitch"], a["pos"], a["tok"], a["B"], a["C"], a["H"], a["W"], a["ph"], a["pw"], a["crop"], 0)
+        _lib.call("cfp_posenc_tokens_nhwc_fwd", a["x"], a["pitch"], a["pos"], a["tok"], a["B"], a["C"], a["H"], a["W"], a["ph"],
+                  a["pw"], a["oy"], a["ox"], a["crop"], a["dtype"], 0)
 
-    for bad, match in ((dict(crop=0), "null pointer"), (dict(x=0), "null pointer"), (dict(pos=0), "null pointer"),
-                       (dict(tok=0), "null pointer"), (dict(B=0), "bad shape"), (dict(H=31), "larger than"),
-                       (dict(W=41), "larger than"), (dict(C=6), "C = 6"), (dict(pitch=130), "pitch 130"),
-                       (dict(C=256), "C = 256")):
+    for bad, match in ((dict(x=0), "null pointer"), (dict(pos=0), "null pointer"), (dict(tok=0), "null pointer"),
+                       (dict(B=0), "bad shape"), (dict(H=31), "larger than"), (dict(W=41), "larger than"),
+                       (dict(oy=1), "host crop offsets"), (dict(ox=2), "host crop offsets"),
+                       (dict(crop=0, ox=7), "outside the 30x40 table"), (dict(dtype=2), "unsupported dtype 2"),
+                       (dict(C=6), "C = 6"), (dict(pitch=130), "pitch 130"), (dict(C=256), "C = 256")):
         with pytest.raises(_lib.CfpError, match=match):
             call(**bad)
 

@@ -75,7 +75,7 @@ def test_conv_fwd_matches_torch(cin, cout, k, H, W, B, bn, may_pad, coff):
     assert (out[..., :coff] == 7.0).all() and (out[..., coff + cout:] == 7.0).all(), "wrote outside its channel slice"
 
 
-def test_upsample_concat_matches_torch():
+def test_bf16_upsample_concat_matches_torch():
     g = torch.Generator().manual_seed(3)
     B, h, w, H, W, c_lo, c_skip, c_out = 2, 13, 17, 26, 34, 256, 136, 400
     lo = torch.randn(B, c_lo, h, w, generator=g)
@@ -84,7 +84,7 @@ def test_upsample_concat_matches_torch():
     out = torch.empty(B, H, W, c_out, device=DEV, dtype=torch.bfloat16)
     with torch.cuda.device(0):
         _lib.call("cfp_upsample_concat", lo_t.data_ptr(), h, w, c_lo, c_lo, skip.to(DEV).data_ptr(), c_skip, out.data_ptr(), B, H, W,
-                  c_out, _lib.stream_ptr())
+                  c_out, _lib.CFP_BF16, _lib.stream_ptr())
     torch.cuda.synchronize()
     up = F.interpolate(lo.bfloat16().float(), size=[H, W], mode="bilinear", align_corners=True)
     want = torch.cat([up, skip], dim=1).permute(0, 2, 3, 1)

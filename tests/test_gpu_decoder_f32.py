@@ -81,7 +81,7 @@ def test_conv_f32_matches_fp64(cin, cout, k, H, W, B, bn, coff):
     assert torch.equal(outs[0], outs[1]), "two launches differ"
 
 
-def test_upsample_concat_f32_matches_torch():
+def test_fp32_upsample_concat_matches_torch():
     g = torch.Generator().manual_seed(3)
     B, h, w, H, W, c_lo, c_skip, c_out = 2, 13, 17, 26, 34, 256, 136, 400
     lo = torch.randn(B, c_lo, h, w, generator=g)
@@ -89,8 +89,8 @@ def test_upsample_concat_f32_matches_torch():
     skip_d = skip.to(DEV)
     out = torch.full((B, H, W, c_out), float("nan"), device=DEV)
     with torch.cuda.device(0):
-        _lib.call("cfp_upsample_concat_f32", nhwc(lo).data_ptr(), h, w, c_lo, c_lo, skip_d.data_ptr(), c_skip, out.data_ptr(), B, H, W,
-                  c_out, _lib.stream_ptr())
+        _lib.call("cfp_upsample_concat", nhwc(lo).data_ptr(), h, w, c_lo, c_lo, skip_d.data_ptr(), c_skip, out.data_ptr(), B, H, W,
+                  c_out, _lib.CFP_F32, _lib.stream_ptr())
     torch.cuda.synchronize()
     up = F.interpolate(lo.double(), size=[H, W], mode="bilinear", align_corners=True)
     want = torch.cat([up, skip.double()], dim=1).permute(0, 2, 3, 1)
@@ -99,7 +99,7 @@ def test_upsample_concat_f32_matches_torch():
     assert (got[..., c_lo + c_skip:] == 0).all()
 
 
-def test_upsample_concat_f32_without_low_resolution_map():
+def test_fp32_upsample_concat_without_low_resolution_map():
     """Decoder.to_nhwc: NCHW feature -> channels-last, zero channels up to the pitch (lo = NULL, c_lo = 0)."""
     g = torch.Generator().manual_seed(4)
     B, C, H, W, cpad = 2, 230, 13, 17, 240
@@ -107,7 +107,8 @@ def test_upsample_concat_f32_without_low_resolution_map():
     skip_d = skip.to(DEV)
     out = torch.full((B, H, W, cpad), float("nan"), device=DEV)
     with torch.cuda.device(0):
-        _lib.call("cfp_upsample_concat_f32", 0, 1, 1, 0, 8, skip_d.data_ptr(), C, out.data_ptr(), B, H, W, cpad, _lib.stream_ptr())
+        _lib.call("cfp_upsample_concat", 0, 1, 1, 0, 8, skip_d.data_ptr(), C, out.data_ptr(), B, H, W, cpad, _lib.CFP_F32,
+                  _lib.stream_ptr())
     torch.cuda.synchronize()
     got = out.cpu()
     assert torch.equal(got[..., :C], skip.permute(0, 2, 3, 1))

@@ -1,5 +1,5 @@
 """The model below the image encoder as one CUDA graph (cfpnet_b200.pipeline.make_graphed_depth): the NHWC positional-encoding
-kernels with device-resident crop offsets against their host-offset siblings, graph replay against the eager sequence
+entry with device-resident crop offsets against the same entry with host offsets, graph replay against the eager sequence
 (histogram encoder -> Decoder.forward_nhwc -> DepthHead.forward_nhwc) on both engines, positional-encoding draws per replay,
 ownership of the memory the graph reads, and the staleness checks that refuse a replay."""
 import gc
@@ -111,23 +111,24 @@ def replay(run, inputs, seed):
 
 
 # ------------------------------------------------------------------------------------------------ kernels
-@pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float32])
-def test_crop_entry_points_equal_host_offset_entry_points(dtype):
+@pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float32], ids=["bf16", "f32"])
+def test_device_crop_equals_host_offsets(dtype):
     """x_pitch > C: x is the first C channels of a wider channels-last buffer, as the decoder's concat buffer is."""
     g = torch.Generator().manual_seed(1)
     B, C, pitch, H, W, pos_h, pos_w = 2, 64, 128, 52, 68, 60, 80
     x = torch.randn(B, H, W, pitch, generator=g).to(DEV, dtype)
     pos = torch.randn(pos_h * pos_w, C, generator=g).to(DEV)
-    host, dev = (("cfp_posenc_tokens_nhwc_f32_fwd", "cfp_posenc_tokens_nhwc_f32_crop_fwd") if dtype == torch.float32
-                 else ("cfp_posenc_tokens_nhwc_fwd", "cfp_posenc_tokens_nhwc_crop_fwd"))
+    code = _lib.dtype_code(dtype)
     for oy, ox in ((0, 0), (3, 5), (7, 1), (pos_h - H, pos_w - W)):
         want = torch.full((B, H * W, C), float("nan"), device=DEV, dtype=dtype)
         got = torch.full((B, H * W, C), float("nan"), device=DEV, dtype=dtype)
         crop = torch.tensor([oy, ox], dtype=torch.int32, device=DEV)
         with torch.cuda.device(0):
             st = _lib.stream_ptr()
-            _lib.call(host, x.data_ptr(), pitch, pos.data_ptr(), want.data_ptr(), B, C, H, W, pos_h, pos_w, oy, ox, st)
-            _lib.call(dev, x.data_ptr(), pitch, pos.data_ptr(), got.data_ptr(), B, C, H, W, pos_h, pos_w, crop.data_ptr(), st)
+            _lib.call("cfp_posenc_tokens_nhwc_fwd", x.data_ptr(), pitch, pos.data_ptr(), want.data_ptr(), B, C, H, W, pos_h, pos_w,
+                      oy, ox, None, code, st)
+            _lib.call("cfp_posenc_tokens_nhwc_fwd", x.data_ptr(), pitch, pos.data_ptr(), got.data_ptr(), B, C, H, W, pos_h, pos_w,
+                      0, 0, crop.data_ptr(), code, st)
         torch.cuda.synchronize()
         assert torch.equal(got, want), (oy, ox)
         ref = x[..., :C].float() + pos.view(pos_h, pos_w, C)[oy:oy + H, ox:ox + W]

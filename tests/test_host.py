@@ -3,6 +3,7 @@ library's symbol table, and loud failure without a GPU.  No compute calls."""
 import ctypes
 import os
 import re
+import subprocess
 
 import numpy as np
 import pytest
@@ -33,6 +34,11 @@ def test_library_exports_every_declared_symbol(lib):
     for name in declared:
         assert hasattr(raw, name), f"{name} declared in include/cfp.h but not exported"
         assert name in _lib.SIGNATURES, f"{name} has no ctypes signature"
+    # ... and the reverse: an entry point removed from the header must not stay exported
+    nm = subprocess.run(["nm", "-D", "--defined-only", _lib.LIB_PATH], capture_output=True, text=True, check=True).stdout
+    exported = set(re.findall(r"^\S+\s+T\s+(cfp_[a-z0-9_]+)$", nm, re.M))
+    assert exported, nm
+    assert not exported - set(declared), f"exported but not declared in include/cfp.h: {sorted(exported - set(declared))}"
     assert lib.cfp_version() == _lib.ABI_VERSION
     assert lib.cfp_last_error() is not None
 
